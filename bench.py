@@ -27,6 +27,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 from stvo_pl_b200 import synth, types as T  # noqa: E402
 
@@ -390,6 +391,8 @@ def run_ours(args):
     value = world * B * args.steps / (ms * 1e-3)
     out = db.download()
     good = int(out["results"]["good"].sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, prev)
 
     # ---------------- per-kernel times and the roofline of the dominant kernel, rank 0 ----------------
     st = db.stage_times(iters=max(5, min(args.steps, 20)))
@@ -621,6 +624,31 @@ def run_ours(args):
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, out, prev):
+    """Writes what the caller of the timed path receives after its last step (plstvo_batch_download: the pose results and the
+    match / inlier arrays) as float64 .npy files, one per array and per field of the results.  Beyond DUMP_LIMIT bytes only a
+    fixed, seeded sample of the frame pairs is written; pairs.npy names them."""
+    res = out["results"]
+    B = len(res)
+    pairs = np.arange(B)
+    values = sum(int(np.prod(res.dtype[k].shape)) for k in res.dtype.names) + 2 * (len(out["m12_pt"]) + len(out["m12_ls"])) / B
+    per_pair = 8 * values
+    if B * per_pair > DUMP_LIMIT:
+        keep = int((DUMP_LIMIT - (1 << 20)) // per_pair)      # 1 MB left for the .npy headers and pairs.npy
+        pairs = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    arrays = {f"results_{k}": res[k][pairs] for k in res.dtype.names}
+    for kind, off in (("pt", prev.pt_off), ("ls", prev.ls_off)):
+        idx = np.concatenate([np.arange(off[p], off[p + 1]) for p in pairs] + [np.zeros(0, np.int64)])
+        arrays[f"m12_{kind}"], arrays[f"inlier_{kind}"] = out[f"m12_{kind}"][idx], out[f"inlier_{kind}"][idx]
+    arrays["pairs"] = pairs
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(a, np.float64))
 
 
 def c5_sweeps(eng, B, iters=20):
@@ -975,7 +1003,11 @@ def main():
                          "(1920x1080, 8000 points + 2000 lines, >= 1024 problems resident, 20 evaluations)")
     ap.add_argument("--kernels-only", action="store_true",
                     help="profiling aid: upload, launch K1 and K2 over the whole batch twice, exit (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs (rank 0) as DIR/<name>.npy (c1 / c2 / c3)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS or args.kernels_only):
+        ap.error("--dump-outputs applies to the c1 / c2 / c3 workloads of --impl ours")
     global ACTIVE
     if args.workload in WORKLOADS:
         ACTIVE = args.workload

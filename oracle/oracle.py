@@ -9,6 +9,7 @@ import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -22,9 +23,11 @@ _SRC = [os.path.join(_HERE, "plstvo_oracle.c"), os.path.join(_HERE, "plstvo_orac
 def _build(out: str, march: str) -> None:
     """Same flags as oracle/Makefile (= the reference's CMakeLists.txt:18 flags)."""
     os.makedirs(os.path.dirname(out), exist_ok=True)
+    tmp = f"{out}.{os.getpid()}.tmp"      # renamed into place: a concurrent loader never sees a half-written library
     cmd = ["gcc", "-O3", f"-march={march}", f"-mtune={'native' if march == 'native' else 'generic'}",
-           "-std=gnu11", "-fPIC", "-ffp-contract=off", "-shared", "-o", out, _SRC[0], "-lm", "-lpthread"]
+           "-std=gnu11", "-fPIC", "-ffp-contract=off", "-shared", "-o", tmp, _SRC[0], "-lm", "-lpthread"]
     subprocess.run(cmd, check=True, capture_output=True)
+    os.replace(tmp, out)
 
 
 def _stale(lib: str) -> bool:
@@ -33,7 +36,9 @@ def _stale(lib: str) -> bool:
 
 def lib_path(native: bool = False) -> str:
     """Portable build (x86-64-v3: AVX2 + POPCNT) travels with the repo; the native build used for the CPU
-    baseline is compiled on the machine that times it (-march=native, the reference's own flag)."""
+    baseline is compiled on the machine that times it (-march=native, the reference's own flag).  That one goes to the
+    system's temporary directory, keyed by the sources and the CPU's flags, so that the benchmark runs from a read-only
+    tree."""
     override = os.environ.get("PLSTVO_ORACLE_LIB")   # e.g. an -fsanitize=address,undefined build (tools/oracle_asan.sh)
     if override:
         return override
@@ -47,9 +52,12 @@ def lib_path(native: bool = False) -> str:
             flags = next((l for l in f if l.startswith("flags")), "")
     except OSError:
         flags = ""
-    tag = hashlib.sha1(flags.encode()).hexdigest()[:10]
-    lib = os.path.join(_HERE, "_native", tag, "libplstvo_oracle.so")
-    if _stale(lib):
+    key = hashlib.sha1(flags.encode())
+    for s in _SRC:
+        with open(s, "rb") as f:
+            key.update(f.read())
+    lib = os.path.join(tempfile.gettempdir(), f"plstvo_oracle_native_{os.getuid()}", key.hexdigest()[:16], "libplstvo_oracle.so")
+    if not os.path.exists(lib):
         _build(lib, "native")
     return lib
 

@@ -15,11 +15,6 @@ from stvo_pl_b200 import types as T
 from . import make_ref
 
 
-def available() -> bool:
-    import os
-    return make_ref.available() or os.path.exists(make_ref.LIB)
-
-
 class Ref:
     def __init__(self):
         self.lib = L = C.CDLL(make_ref.build())

@@ -27,4 +27,11 @@ def engine():
     return Engine()
 
 
+@pytest.fixture
+def ref(request):
+    """The reference's own pose code (oracle/_ref), as recorded for this test in tests/golden/ref_outputs.npz."""
+    import ref_golden
+    return ref_golden.for_test(request.node)
+
+
 GOLDEN = os.path.join(ROOT, "tests", "golden")

@@ -2,7 +2,7 @@
 (src/stereoFrame.cpp:515, :545), residuals within a few ulp of removeOutliers' threshold (src/stereoFrameHandler.cpp:1016,
 :1056 with src/auxiliar.cpp:399-427), and the robust (MAD-scaled) mode with the number of differing inlier flags reported.
 Everything runs through the C-ABI (plstvo_optimize_pose / plstvo_track_batch / plstvo_gn_eval_stream) and is compared
-with the oracle; where oracle/_ref is available the reference's own compiled code is the third party."""
+with the oracle; the reference's own compiled code (as recorded in tests/golden/ref_outputs.npz) is the third party."""
 import numpy as np
 import pytest
 
@@ -29,14 +29,6 @@ def _with_obs(m, obs):
                           ls_sigma2=m.ls_sigma2)
 
 
-def _ref_or_none():
-    try:
-        from oracle import ref as ref_mod
-        return ref_mod.Ref() if ref_mod.available() else None
-    except Exception:
-        return None
-
-
 def _same_pose(a, b, ang_tol=1e-9, tr_tol=1e-8):
     ang, tr = R.pose_error(a["DT"], b["DT"])
     assert ang < ang_tol and tr < tr_tol, (ang, tr)
@@ -54,7 +46,7 @@ def _degenerate(m, rng, frac_v=0.3, frac_h=0.3, frac_z=0.0):
     return _with_lines(m, spl, epl), int(v.sum()), int(h.sum()), int(z.sum())
 
 
-def test_degenerate_previous_segments_through_the_solver(engine, oracle):
+def test_degenerate_previous_segments_through_the_solver(engine, oracle, ref):
     """|dx| < 1 and |dy| < 1 previous-frame segments through plstvo_optimize_pose (K2's pre-computed overlap coefficients
     must reproduce all three branches of lineSegmentOverlap)."""
     cfg = T.kitti_config()
@@ -65,13 +57,11 @@ def test_degenerate_previous_segments_through_the_solver(engine, oracle):
     rc, res_o, ip_o, il_o = oracle.optimize_pose(cam, cfg, deg)
     np.testing.assert_array_equal(ip, ip_o)
     np.testing.assert_array_equal(il, il_o)
-    ref = _ref_or_none()
-    res_r = ref.optimize_pose(cam, cfg, deg)[1] if ref else None
+    res_r = ref.optimize_pose(cam, cfg, deg)[1]
     for p in range(4):
         assert res[p]["good"] == 1
         _same_pose(res[p], res_o[p])
-        if res_r is not None:
-            _same_pose(res[p], res_r[p])
+        _same_pose(res[p], res_r[p])
 
 
 def test_degenerate_segments_through_the_streamed_evaluator(engine, oracle):
@@ -87,7 +77,7 @@ def test_degenerate_segments_through_the_streamed_evaluator(engine, oracle):
         assert abs(e[p] - eo) < 5e-4 * max(1.0, abs(eo))
 
 
-def test_zero_length_previous_segments(engine, oracle):
+def test_zero_length_previous_segments(engine, oracle, ref):
     """A zero-length previous segment divides by l(1) = 0 in the vertical branch (src/stereoFrame.cpp:515-544): the lambdas
     are +-inf (NaN only when the projected end point has exactly the same v), the overlap comes out as 0 or 1.  The GPU
     must take the same route: identical flags and pose, also against the reference's compiled code."""
@@ -99,21 +89,18 @@ def test_zero_length_previous_segments(engine, oracle):
     rc, res_o, ip_o, il_o = oracle.optimize_pose(cam, cfg, deg)
     np.testing.assert_array_equal(ip, ip_o)
     np.testing.assert_array_equal(il, il_o)
-    ref = _ref_or_none()
-    res_r = ref.optimize_pose(cam, cfg, deg)[1] if ref else None
+    res_r = ref.optimize_pose(cam, cfg, deg)[1]
     for p in range(3):
         _same_pose(res[p], res_o[p])
-        if res_r is not None:
-            _same_pose(res[p], res_r[p])
+        _same_pose(res[p], res_r[p])
 
 
-def test_outlier_threshold_adversarial(engine, oracle):
+def test_outlier_threshold_adversarial(engine, oracle, ref):
     """Observations moved along their residual direction so that |r - mean| lands within a few ulp of k * stdv on either
     side: the inlier flags must still be identical (the trimmed mean is a block-parallel sum in K2, a sequential one in the
     reference)."""
     cfg = T.kitti_config()
     m, Tgt, cam, *_ = _matched(oracle, "kitti", 2, cfg, n_pt=700, n_ls=150)
-    ref = _ref_or_none()
     obs = m.pt_pl_obs.copy()
     for p in range(2):
         a, b = int(m.pt_off[p]), int(m.pt_off[p + 1])
@@ -143,9 +130,8 @@ def test_outlier_threshold_adversarial(engine, oracle):
     assert int((ip != ip_o).sum()) == 0 and int((il != il_o).sum()) == 0
     for p in range(2):
         _same_pose(res[p], res_o[p])
-    if ref:
-        rc, res_r, ip_r, il_r = ref.optimize_pose(cam, cfg, adv)
-        assert int((ip != ip_r).sum()) == 0 and int((il != il_r).sum()) == 0
+    rc, res_r, ip_r, il_r = ref.optimize_pose(cam, cfg, adv)
+    assert int((ip != ip_r).sum()) == 0 and int((il != il_r).sum()) == 0
 
 
 def test_robust_mode_flag_differences_are_counted(engine, oracle):

@@ -405,37 +405,32 @@ def test_async_streaming_equals_blocking_call(engine):
         assert pinned[k][2]["results"].tobytes() == ref[k]["results"].tobytes()
 
 
-def test_explicit_lists_c5_size(engine, oracle):
+def test_explicit_lists_c5_size(engine, oracle, ref):
     """C5-size explicit lists (8000 + 2000 per problem) through plstvo_optimize_pose: the streamed solver against the oracle
-    (and, where oracle/_ref is there, against the reference's compiled code)."""
+    and against the reference's compiled code."""
     cfg = T.kitti_config()
     mb, Ts, cam = synth.make_matched_batch("hd", 3)
-    rc, ref, rp, rl = oracle.optimize_pose(cam, cfg, mb)
+    rc, res_o, rp, rl = oracle.optimize_pose(cam, cfg, mb)
     res, ip, il = engine.optimize_pose(cam, cfg, mb)
     for p in range(3):
-        assert res["status"][p] == ref["status"][p] and res["good"][p] == ref["good"][p] == 1
-        ang, tr = R.pose_error(res["DT"][p], ref["DT"][p])
+        assert res["status"][p] == res_o["status"][p] and res["good"][p] == res_o["good"][p] == 1
+        ang, tr = R.pose_error(res["DT"][p], res_o["DT"][p])
         assert ang < TOL_ANG and tr < TOL_TR
         a, b, c, d = mb.pt_off[p], mb.pt_off[p + 1], mb.ls_off[p], mb.ls_off[p + 1]
         flips = _flag_diffs(ip[a:b], rp[a:b]) + _flag_diffs(il[c:d], rl[c:d])
         # same inlier set: the error agrees to the fp32 evaluation's noise; a flag that flipped (a residual within fp32 reach of the
         # removeOutliers threshold) moves it by about one feature's share
-        assert abs(res["err_norm"][p] - ref["err_norm"][p]) < (1e-6 if flips == 0 else 2e-4 * flips)
-        np.testing.assert_allclose(res["DT_cov"][p], ref["DT_cov"][p], rtol=2e-3, atol=1e-12)
+        assert abs(res["err_norm"][p] - res_o["err_norm"][p]) < (1e-6 if flips == 0 else 2e-4 * flips)
+        np.testing.assert_allclose(res["DT_cov"][p], res_o["DT_cov"][p], rtol=2e-3, atol=1e-12)
         ang, tr = R.pose_error(res["DT_opt"][p], Ts[p])
         assert ang < 1e-3 and tr < 1e-2
     n_diff = _flag_diffs(ip, rp) + _flag_diffs(il, rl)
     print(f"streamed solver, explicit C5 lists: {n_diff} of {len(ip) + len(il)} inlier flags differ")
     assert n_diff <= 6
-    try:
-        from oracle import ref as ref_mod
-        if ref_mod.available():
-            rr = ref_mod.Ref().optimize_pose(cam, cfg, mb)[1]
-            for p in range(3):
-                ang, tr = R.pose_error(res["DT"][p], rr["DT"][p])
-                assert ang < TOL_ANG and tr < TOL_TR
-    except ImportError:
-        pass
+    rr = ref.optimize_pose(cam, cfg, mb)[1]
+    for p in range(3):
+        ang, tr = R.pose_error(res["DT"][p], rr["DT"][p])
+        assert ang < TOL_ANG and tr < TOL_TR
 
 
 def test_streamed_solver_is_bit_reproducible(engine):

@@ -3,9 +3,10 @@
 oracle/_ref/libplstvo_ref.so holds optimizeFunctions, optimizeFunctionsRobust, gaussNewtonOptimization[Robust],
 removeOutliers, isGoodSolution, optimizePose (src/stereoFrameHandler.cpp:292-480, 549-962, 988-1067), lineSegmentOverlap
 (src/stereoFrame.cpp:510-616), projection / backProjection (src/pinholeStereoCamera.cpp:221-237), the SE(3) helpers and
-the MAD statistics (src/auxiliar.cpp:29-44, 58-62, 113-197, 353-355, 387-430, 444-460, 556-583) compiled from the text of
-/root/reference by line range (oracle/make_ref.py) against stand-in Eigen headers.  Every comparison below is
-oracle (our restatement, oracle/plstvo_oracle.c) == that library on the same inputs.
+the MAD statistics (src/auxiliar.cpp:29-44, 58-62, 113-197, 353-355, 387-430, 444-460, 556-583) compiled from the original
+project's text by line range (oracle/make_ref.py) against stand-in Eigen headers.  Every comparison below is
+oracle (our restatement, oracle/plstvo_oracle.c) == that library on the same inputs.  The library's outputs are the ones
+recorded in tests/golden/ref_outputs.npz (the `ref` fixture, tests/ref_golden.py).
 
 What the library does NOT contain is Eigen itself: its 6x6 decompositions are the stand-in's, so the first group of tests
 holds those against LAPACK (numpy.linalg) instead.
@@ -15,15 +16,6 @@ import pytest
 
 import ref_numpy as R
 from stvo_pl_b200 import synth, types as T
-
-ref_mod = pytest.importorskip("oracle.ref")
-if not ref_mod.available():
-    pytest.skip("oracle/_ref not built and /root/reference absent", allow_module_level=True)
-
-
-@pytest.fixture(scope="module")
-def ref():
-    return ref_mod.Ref()
 
 
 def _rng(seed):
