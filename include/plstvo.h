@@ -345,19 +345,19 @@ void  plstvo_host_free(void* p);
 /* ---- instrumentation -------------------------------------------------------------------------- */
 /* kernels launched by this library since the context was created (bench.py's gpu_launches) */
 int64_t plstvo_launch_count(const PlContext* ctx);
-/* device time of the two kernels of one pass over the resident batch, each launched alone `iters` times
+/* device time of the two stages of one pass over the resident batch, each launched alone `iters` times
  * on the context's stream and bracketed by CUDA events on that stream: *ms_match / *ms_solve = average
- * duration of one K1 (hamming_knn2 over all tiles of the batch) / one K2 (track_solve, one CTA per pair)
- * launch.  n_tiles / n_pairs (optional) = CTAs per launch. */
+ * duration of one K1 (tc_expand + tc_hamming + tc_resolve over the batch) / one K2 (track_solve, one CTA per pair).
+ * n_tiles (optional) = matching problems with work (enabled, both sides non-empty); n_pairs (optional) = pairs. */
 int     plstvo_batch_kernel_times(PlContext* ctx, PlDeviceBatch* db, int iters, double* ms_match,
                                   double* ms_solve, int32_t* n_tiles, int32_t* n_pairs);
-/* The same per stage: ms[0] = operand expansion, ms[1] = distance + top-2 kernel (tcgen05 form) or the integer K1
- * (PLSTVO_K1=popc: ms[0] = ms[2] = 0), ms[2] = index resolution, ms[3] = building matched_pt / matched_ls when that is a
- * kernel of its own (the streamed solver; 0 when K2 does it internally), ms[4] = optimizePose (K2, or the streamed solver's
+/* The same per stage: ms[0] = operand expansion, ms[1] = distance + top-2 kernel (tcgen05),
+ * ms[2] = index resolution, ms[3] = building matched_pt / matched_ls when that is a kernel of its own (the streamed
+ * solver; 0 when K2 does it internally), ms[4] = optimizePose (K2, or the streamed solver's
  * GN-loop / outlier / finalize kernels + K2 for the problems it hands back); of ms[4], streamed solver only (0 for K2):
  * ms[5] = the GN loop launch of stage 1, ms[6] = the gate + removeOutliers launch, ms[7] = the GN loop launch of stage 2.
  * counts (optional) = {bit 0: tensor-core matcher, bit 1: streamed solver, bits 8..: problems the streamed solver handed to
- * the fp64 kernel in the last pass; work items (or tiles) of the distance kernel; matching problems; pairs}. */
+ * the fp64 kernel in the last pass; work items of the distance kernel; matching problems; pairs}. */
 int     plstvo_batch_stage_times(PlContext* ctx, PlDeviceBatch* db, int iters, double ms[8], int32_t counts[4]);
 /* GN evaluation (optimizeFunctions, src/stereoFrameHandler.cpp:549-694) of the resident matched
  * lists at given poses, streamed from HBM: the roofline kernel of config C5.

@@ -50,9 +50,7 @@ struct Workspace {
     std::vector<int32_t> p_off1, p_off2, l_off1, l_off2;
     // plan
     std::vector<MatchProblem> problems;   // [2B]: points, lines
-    std::vector<MatchTile> tiles;
-    std::vector<int32_t> tile_start;      // [B+1] first tile of each pair
-    int max_tsplit = 32, cap_pt = 0, cap_ls = 0, sort_cap = 1, max_n2 = 0;
+    int cap_pt = 0, cap_ls = 0, sort_cap = 1, max_n2 = 0;
     bool feat_in_smem = true;
     // device storage
     DevBuf d_poff1, d_poff2, d_loff1, d_loff2;
@@ -60,10 +58,9 @@ struct Workspace {
     DevBuf d_ptP, d_pts2, d_ptpl;                                      // prev P, prev sigma2, curr pl
     DevBuf d_lssP, d_lseP, d_lsspl, d_lsepl, d_lss2, d_lslev, d_lsle;  // prev ...; curr le
     DevBuf d_priors, d_results, d_m12p, d_m12l, d_inlp, d_inll;
-    DevBuf d_rowpart, d_colpart, d_problems, d_tiles, d_feat;
+    DevBuf d_rowpart, d_colpart, d_problems, d_feat;
     DevBuf d_phase;   // debug phase timers (PLSTVO_PHASE_DEBUG)
-    // tensor-core form of K1 (match_tc.cu): expanded operands, per-block value partials, work items
-    bool use_tc = true;
+    // K1 on the tensor cores (match_tc.cu): expanded operands, per-block value partials, work items
     std::vector<TcProblem> tc_problems;   // [2B], parallel to `problems`
     std::vector<TcSide> tc_sides;         // [4B]: queries, trains of every problem
     std::vector<TcItem> tc_items[2];      // work items of the point problems (long) and of the line problems (short)
@@ -77,7 +74,7 @@ struct Workspace {
         DevBuf* all[] = {&d_poff1, &d_poff2, &d_loff1, &d_loff2, &d_pdesc1, &d_pdesc2, &d_ldesc1, &d_ldesc2,
                          &d_ptP, &d_pts2, &d_ptpl, &d_lssP, &d_lseP, &d_lsspl, &d_lsepl, &d_lss2, &d_lslev,
                          &d_lsle, &d_priors, &d_results, &d_m12p, &d_m12l, &d_inlp, &d_inll, &d_rowpart,
-                         &d_colpart, &d_problems, &d_tiles, &d_feat, &d_phase, &d_tcprob, &d_tcsides, &d_tcitems[0],
+                         &d_colpart, &d_problems, &d_feat, &d_phase, &d_tcprob, &d_tcsides, &d_tcitems[0],
                          &d_tcitems[1], &d_exp, &d_rowp, &d_colp, &d_sched, &d_stream};
         for (DevBuf* b : all) b->release();
     }
@@ -216,37 +213,12 @@ StreamBufs stream_bufs_at(const StreamBufs& sb, int p0) {
 }
 
 // ---- planning -------------------------------------------------------------------------------------
-// target_ctas: how many K1 tiles we would like at least, so that small batches still fill the chip
-// PLSTVO_K1=popc selects the integer (XOR + POPC) form of K1; the default is the tensor-core form (match_tc.cu)
-bool k1_use_tc() {
-    static const bool tc = [] {
-        const char* v = getenv("PLSTVO_K1");
-        return !(v && !strcmp(v, "popc"));
-    }();
-    return tc;
-}
-
-void plan_problem(MatchProblem& pr, int n1, int n2, bool enabled, float nnr, int best_lr, int tsplit_hint, bool use_tc) {
+void plan_problem(MatchProblem& pr, int n1, int n2, bool enabled, float nnr, int best_lr) {
     pr.n1 = n1;
     pr.n2 = n2;
     pr.nnr = nnr;
     pr.best_lr = best_lr;
     pr.enabled = (enabled && n1 > 0 && n2 > 0) ? 1 : 0;   // src/stereoFrameHandler.cpp:137-138, :160-161
-    if (!pr.enabled) {
-        pr.nqb = pr.ntb = 0;
-        pr.tsplit = 32;
-        return;
-    }
-    if (use_tc) {   // tc_resolve_kernel leaves ONE merged partial per row and per column
-        pr.nqb = pr.ntb = 1;
-        pr.tsplit = 32;
-        return;
-    }
-    pr.nqb = (n1 + k1_queries_per_tile() - 1) / k1_queries_per_tile();
-    int ts = ((n2 + 31) / 32) * 32;
-    if (tsplit_hint > 0 && tsplit_hint < ts) ts = tsplit_hint;
-    pr.tsplit = ts;
-    pr.ntb = (n2 + ts - 1) / ts;
 }
 
 int validate_frames(PlContext* ctx, const PlFrameBatch* prev, const PlFrameBatch* curr, bool need_features) {
@@ -302,7 +274,6 @@ int ws_prepare(PlContext* ctx, Workspace& ws, const PlCamera* cam, const PlConfi
     }
     ws.planned = false;
     ws.B = B;
-    ws.use_tc = k1_use_tc();
     if (cam) ws.cam = *cam;
     ws.cfg = *cfg;
     ws.has_priors = has_priors;
@@ -312,30 +283,12 @@ int ws_prepare(PlContext* ctx, Workspace& ws, const PlCamera* cam, const PlConfi
     ws.l_off2.assign(curr->ls_off, curr->ls_off + B + 1);
     const size_t np1 = ws.p_off1[B], np2 = ws.p_off2[B], nl1 = ws.l_off1[B], nl2 = ws.l_off2[B];
 
-    // --- tile split: enough CTAs for a small batch, whole train sets per tile for a big one ---
-    long base_tiles = 0;
-    for (int p = 0; p < B; ++p) {
-        base_tiles += (ws.p_off1[p + 1] - ws.p_off1[p] + k1_queries_per_tile() - 1) / k1_queries_per_tile();
-        base_tiles += (ws.l_off1[p + 1] - ws.l_off1[p] + k1_queries_per_tile() - 1) / k1_queries_per_tile();
-    }
-    const long want = 3L * ctx->sm_count;   // about one full wave of resident K1 CTAs
-    int split = 1;
-    if (base_tiles > 0 && base_tiles < want) split = (int)((want + base_tiles - 1) / base_tiles);
-    // Big batches too: four train blocks per problem (tiles of 512 queries x ~n2/4 trains, at least 256).  Finer tiles shrink
-    // the tail of the last wave of CTAs (2560 tiles of 0.57 ms on 444 slots = 5.77 waves); measured on C2: K1 3.32 -> 3.12 ms,
-    // 129.0 -> 132.4 K solves/s, the blocking call 99 -> 109 K; beyond 4 the extra partials cost K2 more than K1 gains.
-    static const int forced_split = getenv("PLSTVO_K1_SPLIT") ? atoi(getenv("PLSTVO_K1_SPLIT")) : 0;   // tuning knob
-    split = forced_split > 0 ? forced_split : std::max(split, 4);
-
     ws.problems.assign((size_t)2 * B, MatchProblem{});
-    ws.tiles.clear();
-    ws.tile_start.assign((size_t)B + 1, 0);
-    ws.max_tsplit = 32;
     ws.cap_pt = ws.cap_ls = 0;
     ws.max_n2 = 0;
     size_t row_elems = 0, col_elems = 0, exp_tiles = 0, rowp_elems = 0, colp_elems = 0;
-    ws.tc_problems.assign(ws.use_tc ? (size_t)2 * B : 0, TcProblem{});
-    ws.tc_sides.assign(ws.use_tc ? (size_t)4 * B : 0, TcSide{});
+    ws.tc_problems.assign((size_t)2 * B, TcProblem{});
+    ws.tc_sides.assign((size_t)4 * B, TcSide{});
     for (int k = 0; k < 2; ++k) {
         ws.tc_items[k].clear();
         ws.item_start[k].assign((size_t)B + 1, 0);
@@ -343,52 +296,40 @@ int ws_prepare(PlContext* ctx, Workspace& ws, const PlCamera* cam, const PlConfi
     ws.tc_max_tiles = 0;
     const float nnr_p = (float)cfg->min_ratio_12_p, nnr_l = (float)cfg->min_ratio_12_l;   // double -> float at the call
     for (int p = 0; p < B; ++p) {
-        ws.tile_start[p] = (int32_t)ws.tiles.size();
         ws.item_start[0][p] = (int32_t)ws.tc_items[0].size();
         ws.item_start[1][p] = (int32_t)ws.tc_items[1].size();
         for (int type = 0; type < 2; ++type) {
             MatchProblem& pr = ws.problems[(size_t)2 * p + type];
             const int n1 = type ? ws.l_off1[p + 1] - ws.l_off1[p] : ws.p_off1[p + 1] - ws.p_off1[p];
             const int n2 = type ? ws.l_off2[p + 1] - ws.l_off2[p] : ws.p_off2[p + 1] - ws.p_off2[p];
-            int hint = 0;
-            if (split > 1) {
-                hint = ((n2 + split - 1) / split + 31) / 32 * 32;
-                if (hint < 256) hint = 256;
-            }
             plan_problem(pr, n1, n2, type ? cfg->has_lines != 0 : cfg->has_points != 0, type ? nnr_l : nnr_p,
-                         cfg->best_lr_matches != 0, hint, ws.use_tc);
-            if (ws.use_tc) {
-                // operands and partials as element / tile indices first, fixed up after allocation
-                const int t1 = pr.enabled ? (n1 + TC_ROWS - 1) / TC_ROWS : 0, t2 = pr.enabled ? (n2 + TC_ROWS - 1) / TC_ROWS : 0;
-                TcProblem& tp = ws.tc_problems[(size_t)2 * p + type];
-                tp.n1 = n1;
-                tp.n2 = n2;
-                tp.xe = reinterpret_cast<const uint8_t*>(exp_tiles);
-                tp.ye = reinterpret_cast<const uint8_t*>(exp_tiles + t1);
-                tp.rowp = reinterpret_cast<uint32_t*>(rowp_elems);
-                tp.colp = reinterpret_cast<uint32_t*>(colp_elems);
-                ws.tc_sides[(size_t)4 * p + 2 * type] = TcSide{nullptr, pr.enabled ? n1 : 0, nullptr};
-                ws.tc_sides[(size_t)4 * p + 2 * type + 1] = TcSide{nullptr, pr.enabled ? n2 : 0, nullptr};
-                exp_tiles += (size_t)t1 + t2;
-                rowp_elems += (size_t)(pr.enabled ? (n2 + TC_CW - 1) / TC_CW : 0) * n1;
-                colp_elems += (size_t)(pr.enabled ? n2 : 0);
-                ws.tc_max_tiles = std::max(ws.tc_max_tiles, std::max(t1, t2));
-                for (int yb = 0; yb < (t2 + 1) / 2; ++yb) ws.tc_items[type].push_back(TcItem{2 * p + type, yb});
-            }
-            // offsets into the partial buffers are stored as element indices first, fixed up after allocation
+                         cfg->best_lr_matches != 0);
+            // operands and partials as element / tile indices first, fixed up after allocation
+            const int t1 = pr.enabled ? (n1 + TC_ROWS - 1) / TC_ROWS : 0, t2 = pr.enabled ? (n2 + TC_ROWS - 1) / TC_ROWS : 0;
+            TcProblem& tp = ws.tc_problems[(size_t)2 * p + type];
+            tp.n1 = n1;
+            tp.n2 = n2;
+            tp.xe = reinterpret_cast<const uint8_t*>(exp_tiles);
+            tp.ye = reinterpret_cast<const uint8_t*>(exp_tiles + t1);
+            tp.rowp = reinterpret_cast<uint32_t*>(rowp_elems);
+            tp.colp = reinterpret_cast<uint32_t*>(colp_elems);
+            ws.tc_sides[(size_t)4 * p + 2 * type] = TcSide{nullptr, pr.enabled ? n1 : 0, nullptr};
+            ws.tc_sides[(size_t)4 * p + 2 * type + 1] = TcSide{nullptr, pr.enabled ? n2 : 0, nullptr};
+            exp_tiles += (size_t)t1 + t2;
+            rowp_elems += (size_t)(pr.enabled ? (n2 + TC_CW - 1) / TC_CW : 0) * n1;
+            colp_elems += (size_t)(pr.enabled ? n2 : 0);
+            ws.tc_max_tiles = std::max(ws.tc_max_tiles, std::max(t1, t2));
+            for (int yb = 0; yb < (t2 + 1) / 2; ++yb) ws.tc_items[type].push_back(TcItem{2 * p + type, yb});
+            // one merged key pair per row and per column (tc_resolve_kernel), also as element indices first
             pr.rowpart = reinterpret_cast<uint2*>(row_elems);
             pr.colpart = reinterpret_cast<uint2*>(col_elems);
-            row_elems += (size_t)pr.ntb * n1;
-            col_elems += (size_t)pr.nqb * n2;
-            for (int qb = 0; qb < pr.nqb; ++qb)
-                for (int tb = 0; tb < pr.ntb; ++tb) ws.tiles.push_back(MatchTile{2 * p + type, qb, tb});
-            if (pr.enabled) ws.max_tsplit = std::max(ws.max_tsplit, pr.tsplit);
+            row_elems += (size_t)(pr.enabled ? n1 : 0);
+            col_elems += (size_t)(pr.enabled ? n2 : 0);
             ws.max_n2 = std::max(ws.max_n2, n2);
             if (type == 0) ws.cap_pt = std::max(ws.cap_pt, n1);
             else ws.cap_ls = std::max(ws.cap_ls, n1);
         }
     }
-    ws.tile_start[B] = (int32_t)ws.tiles.size();
     ws.item_start[0][B] = (int32_t)ws.tc_items[0].size();
     ws.item_start[1][B] = (int32_t)ws.tc_items[1].size();
     ws.cap_pt = std::max(ws.cap_pt, 1);
@@ -402,8 +343,6 @@ int ws_prepare(PlContext* ctx, Workspace& ws, const PlCamera* cam, const PlConfi
     // PLSTVO_MAX_FEATURES rows
     if (with_features && !ws.feat_in_smem && k2_smem_bytes(ws.cap_pt, ws.cap_ls, ws.sort_cap, false) > ctx->smem_optin)
         return fail(ctx, PLSTVO_E_TOO_LARGE, "frame too large for the per-pair solver's shared memory");
-    if (!ws.use_tc && k1_smem_bytes(ws.max_tsplit) > ctx->smem_optin)
-        return fail(ctx, PLSTVO_E_TOO_LARGE, "train set too large for one K1 tile");
 
     // --- device storage ---
     CK(ctx, ws.d_pdesc1.ensure(np1 * 32));
@@ -415,18 +354,15 @@ int ws_prepare(PlContext* ctx, Workspace& ws, const PlCamera* cam, const PlConfi
     CK(ctx, ws.d_rowpart.ensure(row_elems * sizeof(uint2)));
     CK(ctx, ws.d_colpart.ensure(col_elems * sizeof(uint2)));
     CK(ctx, ws.d_problems.ensure(ws.problems.size() * sizeof(MatchProblem)));
-    CK(ctx, ws.d_tiles.ensure(ws.tiles.size() * sizeof(MatchTile)));
-    if (ws.use_tc) {
-        CK(ctx, ws.d_exp.ensure(exp_tiles * TC_TILE_BYTES + 1024));
-        CK(ctx, ws.d_rowp.ensure(rowp_elems * sizeof(uint32_t)));
-        CK(ctx, ws.d_colp.ensure(colp_elems * sizeof(uint32_t)));
-        CK(ctx, ws.d_tcprob.ensure(ws.tc_problems.size() * sizeof(TcProblem)));
-        CK(ctx, ws.d_tcsides.ensure(ws.tc_sides.size() * sizeof(TcSide)));
-        for (int k = 0; k < 2; ++k) CK(ctx, ws.d_tcitems[k].ensure(ws.tc_items[k].size() * sizeof(TcItem)));
-        if (!ws.d_sched.p) {   // scheduler words of the persistent matcher: one pair per compute stream, self re-arming
-            CK(ctx, ws.d_sched.ensure(64));
-            CK(ctx, cudaMemsetAsync(ws.d_sched.p, 0, 64, ctx->s_h2d));
-        }
+    CK(ctx, ws.d_exp.ensure(exp_tiles * TC_TILE_BYTES + 1024));
+    CK(ctx, ws.d_rowp.ensure(rowp_elems * sizeof(uint32_t)));
+    CK(ctx, ws.d_colp.ensure(colp_elems * sizeof(uint32_t)));
+    CK(ctx, ws.d_tcprob.ensure(ws.tc_problems.size() * sizeof(TcProblem)));
+    CK(ctx, ws.d_tcsides.ensure(ws.tc_sides.size() * sizeof(TcSide)));
+    for (int k = 0; k < 2; ++k) CK(ctx, ws.d_tcitems[k].ensure(ws.tc_items[k].size() * sizeof(TcItem)));
+    if (!ws.d_sched.p) {   // scheduler words of the persistent matcher: one pair per compute stream, self re-arming
+        CK(ctx, ws.d_sched.ensure(64));
+        CK(ctx, cudaMemsetAsync(ws.d_sched.p, 0, 64, ctx->s_h2d));
     }
     if (with_features) {
         CK(ctx, ws.d_poff1.ensure((B + 1) * 4));
@@ -470,23 +406,21 @@ int ws_prepare(PlContext* ctx, Workspace& ws, const PlCamera* cam, const PlConfi
                 pr.d2 = ws.d_ldesc2.as<uint8_t>() + (size_t)ws.l_off2[p] * 32;
                 pr.m12 = ws.d_m12l.as<int32_t>() + ws.l_off1[p];
             }
-            if (ws.use_tc) {
-                TcProblem& tp = ws.tc_problems[(size_t)2 * p + type];
-                uint8_t* ebase = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws.d_exp.p) + 1023) & ~(uintptr_t)1023);
-                uint8_t* xe = ebase + reinterpret_cast<size_t>(tp.xe) * TC_TILE_BYTES;
-                uint8_t* ye = ebase + reinterpret_cast<size_t>(tp.ye) * TC_TILE_BYTES;
-                tp.xe = xe;
-                tp.ye = ye;
-                tp.rowp = ws.d_rowp.as<uint32_t>() + reinterpret_cast<size_t>(tp.rowp);
-                tp.colp = ws.d_colp.as<uint32_t>() + reinterpret_cast<size_t>(tp.colp);
-                ws.tc_sides[(size_t)4 * p + 2 * type].src = pr.d1;
-                ws.tc_sides[(size_t)4 * p + 2 * type].dst = xe;
-                ws.tc_sides[(size_t)4 * p + 2 * type + 1].src = pr.d2;
-                ws.tc_sides[(size_t)4 * p + 2 * type + 1].dst = ye;
-            }
+            TcProblem& tp = ws.tc_problems[(size_t)2 * p + type];
+            uint8_t* ebase = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws.d_exp.p) + 1023) & ~(uintptr_t)1023);
+            uint8_t* xe = ebase + reinterpret_cast<size_t>(tp.xe) * TC_TILE_BYTES;
+            uint8_t* ye = ebase + reinterpret_cast<size_t>(tp.ye) * TC_TILE_BYTES;
+            tp.xe = xe;
+            tp.ye = ye;
+            tp.rowp = ws.d_rowp.as<uint32_t>() + reinterpret_cast<size_t>(tp.rowp);
+            tp.colp = ws.d_colp.as<uint32_t>() + reinterpret_cast<size_t>(tp.colp);
+            ws.tc_sides[(size_t)4 * p + 2 * type].src = pr.d1;
+            ws.tc_sides[(size_t)4 * p + 2 * type].dst = xe;
+            ws.tc_sides[(size_t)4 * p + 2 * type + 1].src = pr.d2;
+            ws.tc_sides[(size_t)4 * p + 2 * type + 1].dst = ye;
         }
     cudaStream_t s = ctx->s_h2d;
-    if (ws.use_tc && !ws.tc_problems.empty()) {
+    if (!ws.tc_problems.empty()) {
         CK(ctx, cudaMemcpyAsync(ws.d_tcprob.p, ws.tc_problems.data(), ws.tc_problems.size() * sizeof(TcProblem),
                                 cudaMemcpyHostToDevice, s));
         CK(ctx, cudaMemcpyAsync(ws.d_tcsides.p, ws.tc_sides.data(), ws.tc_sides.size() * sizeof(TcSide),
@@ -498,9 +432,6 @@ int ws_prepare(PlContext* ctx, Workspace& ws, const PlCamera* cam, const PlConfi
     }
     if (!ws.problems.empty())
         CK(ctx, cudaMemcpyAsync(ws.d_problems.p, ws.problems.data(), ws.problems.size() * sizeof(MatchProblem),
-                                cudaMemcpyHostToDevice, s));
-    if (!ws.tiles.empty())
-        CK(ctx, cudaMemcpyAsync(ws.d_tiles.p, ws.tiles.data(), ws.tiles.size() * sizeof(MatchTile),
                                 cudaMemcpyHostToDevice, s));
     if (with_features) {
         CK(ctx, cudaMemcpyAsync(ws.d_poff1.p, ws.p_off1.data(), (B + 1) * 4, cudaMemcpyHostToDevice, s));
@@ -548,27 +479,18 @@ int ws_upload_range(PlContext* ctx, Workspace& ws, const PlFrameBatch* prev, con
 }
 
 int ws_launch_match(PlContext* ctx, Workspace& ws, int p0, int p1, cudaStream_t s, cudaEvent_t* marks = nullptr) {
-    if (ws.use_tc) {
-        const int a0 = ws.item_start[0][p0], a1 = ws.item_start[0][p1], b0 = ws.item_start[1][p0], b1 = ws.item_start[1][p1];
-        if (a1 > a0 || b1 > b0) {
-            CK(ctx, launch_tc_expand(ws.d_tcsides.as<TcSide>() + (size_t)4 * p0, 4 * (p1 - p0), ws.tc_max_tiles, s));
-            if (marks) CK(ctx, cudaEventRecord(marks[0], s));
-            // launches on the two compute streams may overlap: each has its own pair of scheduler words
-            int* sched = ws.d_sched.as<int>() + (s == ctx->s_alt ? 8 : 0);
-            CK(ctx, launch_tc_hamming(ws.d_tcprob.as<TcProblem>(), ws.d_tcitems[0].as<TcItem>() + a0, a1 - a0,
-                                      ws.d_tcitems[1].as<TcItem>() + b0, b1 - b0, sched, ctx->sm_count, nullptr, s));
-            if (marks) CK(ctx, cudaEventRecord(marks[1], s));
-            CK(ctx, launch_tc_resolve(ws.d_problems.as<MatchProblem>() + (size_t)2 * p0, ws.d_tcprob.as<TcProblem>() + (size_t)2 * p0,
-                                      2 * (p1 - p0), 4, s));
-            ctx->launches += 3;
-        }
-        return 0;
-    }
-    const int t0 = ws.tile_start[p0], t1 = ws.tile_start[p1];
-    if (t1 > t0) {
-        CK(ctx, launch_hamming_knn2(ws.d_problems.as<MatchProblem>(), ws.d_tiles.as<MatchTile>() + t0, t1 - t0,
-                                    ws.max_tsplit, s));
-        ctx->launches++;
+    const int a0 = ws.item_start[0][p0], a1 = ws.item_start[0][p1], b0 = ws.item_start[1][p0], b1 = ws.item_start[1][p1];
+    if (a1 > a0 || b1 > b0) {
+        CK(ctx, launch_tc_expand(ws.d_tcsides.as<TcSide>() + (size_t)4 * p0, 4 * (p1 - p0), ws.tc_max_tiles, s));
+        if (marks) CK(ctx, cudaEventRecord(marks[0], s));
+        // launches on the two compute streams may overlap: each has its own pair of scheduler words
+        int* sched = ws.d_sched.as<int>() + (s == ctx->s_alt ? 8 : 0);
+        CK(ctx, launch_tc_hamming(ws.d_tcprob.as<TcProblem>(), ws.d_tcitems[0].as<TcItem>() + a0, a1 - a0,
+                                  ws.d_tcitems[1].as<TcItem>() + b0, b1 - b0, sched, ctx->sm_count, nullptr, s));
+        if (marks) CK(ctx, cudaEventRecord(marks[1], s));
+        CK(ctx, launch_tc_resolve(ws.d_problems.as<MatchProblem>() + (size_t)2 * p0, ws.d_tcprob.as<TcProblem>() + (size_t)2 * p0,
+                                  2 * (p1 - p0), 4, s));
+        ctx->launches += 3;
     }
     return 0;
 }
@@ -1889,7 +1811,9 @@ int plstvo_batch_kernel_times(PlContext* ctx, PlDeviceBatch* db, int iters, doub
     }
     if (ms_match) *ms_match = tm / iters;
     if (ms_solve) *ms_solve = tsv / iters;
-    if (n_tiles) *n_tiles = (int32_t)ws.tiles.size();
+    if (n_tiles)   // one tile per enabled matching problem
+        *n_tiles = (int32_t)std::count_if(ws.problems.begin(), ws.problems.end(),
+                                          [](const MatchProblem& pr) { return pr.enabled != 0; });
     if (n_pairs) *n_pairs = ws.B;
     return 0;
 }
@@ -1906,10 +1830,8 @@ int plstvo_batch_stage_times(PlContext* ctx, PlDeviceBatch* db, int iters, doubl
     double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     for (int i = 0; i < iters; ++i) {
         CK(ctx, cudaEventRecord(ev[0], ctx->s_main));
-        if (!ws.use_tc) CK(ctx, cudaEventRecord(ev[1], ctx->s_main));   // the integer form is one kernel: reported in slot 1
-        int rc = ws_launch_match(ctx, ws, 0, ws.B, ctx->s_main, ws.use_tc ? &ev[1] : nullptr);
+        int rc = ws_launch_match(ctx, ws, 0, ws.B, ctx->s_main, &ev[1]);
         if (rc) return rc;
-        if (!ws.use_tc) CK(ctx, cudaEventRecord(ev[2], ctx->s_main));
         CK(ctx, cudaEventRecord(ev[3], ctx->s_main));
         rc = ws_launch_solve(ctx, ws, 0, ws.B, ws.have_level, ctx->s_main, &ev[4]);
         if (rc) return rc;
@@ -1937,8 +1859,8 @@ int plstvo_batch_stage_times(PlContext* ctx, PlDeviceBatch* db, int iters, doubl
             CK(ctx, cudaMemcpy(act.data(), sb.active, (size_t)ws.B * sizeof(int32_t), cudaMemcpyDeviceToHost));
             for (int32_t a : act) delegated += a != 0;
         }
-        counts[0] = (ws.use_tc ? 1 : 0) | (ws.use_stream ? 2 : 0) | (delegated << 8);
-        counts[1] = ws.use_tc ? (int32_t)(ws.tc_items[0].size() + ws.tc_items[1].size()) : (int32_t)ws.tiles.size();
+        counts[0] = 1 | (ws.use_stream ? 2 : 0) | (delegated << 8);   // bit 0: tensor-core matcher (always)
+        counts[1] = (int32_t)(ws.tc_items[0].size() + ws.tc_items[1].size());
         counts[2] = (int32_t)ws.problems.size();
         counts[3] = ws.B;
     }

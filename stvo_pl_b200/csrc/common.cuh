@@ -13,34 +13,21 @@ namespace plstvo {
 
 constexpr uint32_t KEY_NONE = 0xFFFFFFFFu;  // "no neighbour": larger than any (dist << 16 | idx) key
 
-// ---- K1 (hamming_knn2) work description -----------------------------------------------------------
+// ---- K1 (tensor-core matcher, match_tc.cu) result description --------------------------------------
 // One matching problem = StVO::match(desc1, desc2) for one feature type of one frame pair
-// (src/matching.cpp:63-91).  The N1 x N2 distance matrix is cut into nqb x ntb tiles; every tile emits
-// a row partial (top-2 over its trains for each of its queries) and a column partial (top-2 over its
-// queries for each of its trains): both directions of the mutual check from ONE pass over the distances.
+// (src/matching.cpp:63-91).  K1 leaves one merged key pair per row (top-2 trains of each query) and one per
+// column (top-2 queries of each train): both directions of the mutual check from ONE pass over the distances.
 struct MatchProblem {
     const uint8_t* d1;     // [n1][32]
     const uint8_t* d2;     // [n2][32]
     int32_t n1, n2;
-    int32_t nqb, ntb;      // tiles along queries / trains
-    int32_t tsplit;        // trains per tile (multiple of 32)
-    int32_t enabled;       // 0: Config::hasPoints()/hasLines() false or an empty side -> all -1, no tiles
-    uint2*  rowpart;       // [ntb][n1]  (k1,k2) packed keys (dist << 16 | train index)
-    uint2*  colpart;       // [nqb][n2]  (k1,k2) packed keys (dist << 16 | query index)
+    int32_t enabled;       // 0: Config::hasPoints()/hasLines() false or an empty side -> all -1, no matching
+    uint2*  rowpart;       // [n1]  (k1,k2) packed keys (dist << 16 | train index)
+    uint2*  colpart;       // [n2]  (k1,k2) packed keys (dist << 16 | query index)
     int32_t* m12;          // [n1] result (problem-local train index or -1)
     float   nnr;
     int32_t best_lr;
 };
-
-struct MatchTile {
-    int32_t problem;
-    int32_t qb;
-    int32_t tb;
-};
-
-constexpr int K1_THREADS = 256;
-int k1_queries_per_tile();                         // K1_THREADS x (query descriptors per thread: 2 or 4), see match.cu
-constexpr int K1_CHUNK   = 512;                    // train rows per TMA stage (16 KB)
 
 // ---- K2 (track_solve) ------------------------------------------------------------------------------
 constexpr int K2_THREADS = 512;   // one pair per SM at a time: at a few pairs per SM the per-pair latency is what counts
@@ -139,8 +126,6 @@ size_t k2_smem_bytes(int cap_pt, int cap_ls, int sort_cap, bool feat_in_smem);
 size_t k2_feat_stride(int cap_pt, int cap_ls);   // doubles of global feature scratch per pair
 
 // kernel launchers (defined in match.cu / solve.cu)
-cudaError_t launch_hamming_knn2(const MatchProblem* problems, const MatchTile* tiles, int n_tiles,
-                                int max_tsplit, cudaStream_t stream);
 cudaError_t launch_match_finalize(const MatchProblem* problems, int n_problems, int max_n2, int32_t* counts,
                                   cudaStream_t stream);
 cudaError_t launch_track_solve(const SolveParams& prm, int n_pairs, cudaStream_t stream);
@@ -149,7 +134,6 @@ cudaError_t launch_select_selftest(const double* v, const int32_t* off, const in
 cudaError_t launch_algebra_selftest(const double* H, const double* g, int n, double* x, double* lad, double* inv,
                                     double* eig, cudaStream_t stream);
 cudaError_t launch_popc_bench(uint32_t* out, int iters, int blocks, cudaStream_t stream);
-size_t k1_smem_bytes(int max_tsplit);
 
 // ---- StVO::matchGrid (match_grid.cu) ---------------------------------------------------------------------------
 struct GridProblem {          // one frame: queries = left image, trains = right image

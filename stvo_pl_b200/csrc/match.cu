@@ -1,231 +1,12 @@
-// match.cu — K1: brute-force 256-bit Hamming 2-NN over descriptor tiles (sm_100a).
+// match.cu — the standalone match finalize and the POPC issue-rate micro-benchmark (sm_100a).
 //
-// Replaces the arithmetic of StVO::matchNNR / StVO::match (src/matching.cpp:41-91), i.e. OpenCV's
-// cv::BFMatcher(NORM_HAMMING)::knnMatch(desc1, desc2, ., 2) called once per direction.  One pass over the
-// N1 x N2 distance matrix produces BOTH directions:
-//   row    top-2 (query  -> nearest trains)  kept in registers, two query descriptors per thread;
-//   column top-2 (train  -> nearest queries) by two warp REDUX.MIN per (warp, train) on packed keys,
-//   merged across warps with shared-memory atomicMin.
-// Keys are (distance << 16 | index): unsigned min == OpenCV's ordering by (distance, trainIdx) ascending,
-// lowest index wins ties for the first and the second neighbour (SURVEY 8(c) probe; golden vectors in
-// tests/golden/match_*.npz).  Train descriptor rows are staged into shared memory by the TMA engine
-// (cp.async.bulk + mbarrier, double buffered); every thread then reads the same row (broadcast LDS.128).
-//
-// Integer work only: XOR + carry-save adders (LOP3) + POPC + IMAD.  No tensor cores: there is no dense
-// contraction here.
-#include <cstdlib>
-
+// match_finalize_kernel: one CTA per matching problem runs match_finalize_block (ratio test + mutual filter,
+// match_finalize.cuh) on the partials K1 (match_tc.cu) left and counts the matches.  plstvo_match_batch and
+// plstvo_f2f_tracking call it; in track mode K2 (solve.cu) runs the same block function itself.
 #include "common.cuh"
 #include "match_finalize.cuh"
 
 namespace plstvo {
-
-constexpr int K1_WARPS = K1_THREADS / 32;
-
-size_t k1_smem_bytes(int max_tsplit) {
-    return 2 * (size_t)K1_CHUNK * 32 + (size_t)max_tsplit * sizeof(uint2) + (size_t)K1_WARPS * 32 * sizeof(uint2) + 64;
-}
-
-__device__ __forceinline__ uint32_t xor3(uint32_t a, uint32_t b, uint32_t c) {
-    uint32_t d;
-    asm("lop3.b32 %0, %1, %2, %3, 0x96;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-__device__ __forceinline__ uint32_t maj3(uint32_t a, uint32_t b, uint32_t c) {
-    uint32_t d;
-    asm("lop3.b32 %0, %1, %2, %3, 0xE8;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-
-// Hamming distance of two 256-bit rows, already shifted into the key's distance field (d << 16).
-// POPC issues at 16 lanes/clk/SM on the XU pipe, LOP3 at 64 on the ALU pipe: three carry-save adders (6 LOP3)
-// fold the eight XOR words into five, so 5 POPC instead of 8 per distance and the two pipes end up balanced.
-//   x0+x1+x2 = s0 + 2 c0,  x3+x4+x5 = s1 + 2 c1,  s0+s1+x6 = s2 + 2 c2   (bitwise, per bit position)
-//   popc(x0..x7) = popc(s2) + popc(x7) + 2 (popc(c0) + popc(c1) + popc(c2))
-template <int NPOPC>
-__device__ __forceinline__ uint32_t hamming256_shl16(const uint4& qa, const uint4& qb, const uint4& a, const uint4& b) {
-    const uint32_t x0 = qa.x ^ a.x, x1 = qa.y ^ a.y, x2 = qa.z ^ a.z, x3 = qa.w ^ a.w;
-    const uint32_t x4 = qb.x ^ b.x, x5 = qb.y ^ b.y, x6 = qb.z ^ b.z, x7 = qb.w ^ b.w;
-    const uint32_t s0 = xor3(x0, x1, x2), c0 = maj3(x0, x1, x2);
-    const uint32_t s1 = xor3(x3, x4, x5), c1 = maj3(x3, x4, x5);
-    if (NPOPC == 6) {   // two adders: 6 POPC, 4 LOP3
-        const uint32_t ones = __popc(s0) + __popc(s1) + __popc(x6) + __popc(x7);
-        const uint32_t twos = __popc(c0) + __popc(c1);
-        return ones * 65536u + twos * 131072u;
-    }
-    const uint32_t s2 = xor3(s0, s1, x6), c2 = maj3(s0, s1, x6);
-    if (NPOPC == 5) {   // three adders: 5 POPC, 6 LOP3
-        const uint32_t ones = __popc(s2) + __popc(x7);
-        const uint32_t twos = __popc(c0) + __popc(c1) + __popc(c2);
-        return ones * 65536u + twos * 131072u;   // IMAD: stays off the ALU pipe
-    }
-    // four adders: 4 POPC, 8 LOP3  (c0 + c1 + c2 = s3 + 2 c3)
-    const uint32_t s3 = xor3(c0, c1, c2), c3 = maj3(c0, c1, c2);
-    const uint32_t ones = __popc(s2) + __popc(x7);
-    return ones * 65536u + __popc(s3) * 131072u + __popc(c3) * 262144u;
-}
-
-template <int NPOPC, int MINB, int QPT>
-__global__ void __launch_bounds__(K1_THREADS, MINB)
-hamming_knn2_kernel(const MatchProblem* __restrict__ problems, const MatchTile* __restrict__ tiles) {
-    constexpr int QTILE = K1_THREADS * QPT;
-    extern __shared__ __align__(128) uint8_t smem[];
-    const MatchTile tile = tiles[blockIdx.x];
-    const MatchProblem pr = problems[tile.problem];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-
-    uint4* stage0 = reinterpret_cast<uint4*>(smem);
-    uint4* stage1 = reinterpret_cast<uint4*>(smem + (size_t)K1_CHUNK * 32);
-    uint2* col = reinterpret_cast<uint2*>(smem + 2 * (size_t)K1_CHUNK * 32);
-    uint2* wstage = col + pr.tsplit + (size_t)warp * 32;    // this warp's column results of the current 32 trains
-    uint64_t* bars = reinterpret_cast<uint64_t*>(col + pr.tsplit + (size_t)K1_WARPS * 32);
-
-    const int t0 = tile.tb * pr.tsplit;
-    const int nt = min(pr.tsplit, pr.n2 - t0);
-
-    // QPT query rows per thread: q, q + K1_THREADS, ... (consecutive lanes -> consecutive rows: coalesced)
-    uint4 qa[QPT], qb[QPT];
-    uint32_t qkey[QPT];
-#pragma unroll
-    for (int u = 0; u < QPT; ++u) {
-        const int q = tile.qb * QTILE + u * K1_THREADS + tid;
-        qa[u] = make_uint4(0, 0, 0, 0);
-        qb[u] = qa[u];
-        qkey[u] = KEY_NONE;   // invalid rows: OR-ing this saturates the column key
-        if (q < pr.n1) {
-            const uint4* p = reinterpret_cast<const uint4*>(pr.d1 + (size_t)q * 32);
-            qa[u] = __ldg(p);
-            qb[u] = __ldg(p + 1);
-            qkey[u] = (uint32_t)q;
-        }
-    }
-    for (int i = tid; i < nt; i += K1_THREADS) col[i] = make_uint2(KEY_NONE, KEY_NONE);
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);
-        mbar_init(&bars[1], 1);
-        fence_mbar_init();
-    }
-    __syncthreads();
-
-    const int nchunks = (nt + K1_CHUNK - 1) / K1_CHUNK;
-    const uint8_t* src = pr.d2 + (size_t)t0 * 32;
-    if (tid == 0) {
-        const uint32_t bytes = (uint32_t)min(K1_CHUNK, nt) * 32u;
-        mbar_arrive_expect_tx(&bars[0], bytes);
-        bulk_g2s(stage0, src, bytes, &bars[0]);
-    }
-
-    uint32_t k1[QPT], k2[QPT];
-#pragma unroll
-    for (int u = 0; u < QPT; ++u) k1[u] = k2[u] = KEY_NONE;
-
-    for (int c = 0; c < nchunks; ++c) {
-        if (tid == 0 && c + 1 < nchunks) {  // prefetch the next stage (its buffer was released by the
-            const int rows = min(K1_CHUNK, nt - (c + 1) * K1_CHUNK);  // __syncthreads of iteration c-1)
-            uint64_t* bar = &bars[(c + 1) & 1];
-            mbar_arrive_expect_tx(bar, (uint32_t)rows * 32u);
-            bulk_g2s(((c + 1) & 1) ? stage1 : stage0, src + (size_t)(c + 1) * K1_CHUNK * 32, (uint32_t)rows * 32u, bar);
-        }
-        mbar_wait(&bars[c & 1], (uint32_t)((c >> 1) & 1));
-        const uint4* s = (c & 1) ? stage1 : stage0;
-        const int cn = min(K1_CHUNK, nt - c * K1_CHUNK);
-        const uint32_t tbase = (uint32_t)(t0 + c * K1_CHUNK);
-
-        for (int g = 0; g < cn; g += 32) {
-            const int gn = min(32, cn - g);
-#pragma unroll 4
-            for (int j = 0; j < gn; ++j) {
-                const uint4 a = s[(g + j) * 2], b = s[(g + j) * 2 + 1];   // same row for every lane: broadcast
-                const uint32_t tkey = tbase + (uint32_t)(g + j);
-                uint32_t kc[QPT];
-#pragma unroll
-                for (int u = 0; u < QPT; ++u) {
-                    const uint32_t dsh = hamming256_shl16<NPOPC>(qa[u], qb[u], a, b);
-                    // row direction: query u of this thread against train tkey
-                    const uint32_t key = dsh | tkey;
-                    k2[u] = min(k2[u], max(k1[u], key));
-                    k1[u] = min(k1[u], key);
-                    kc[u] = dsh | qkey[u];
-                }
-                // column direction: this train against the warp's 32 * QPT queries.  Thread-local top-2, then two
-                // warp REDUX.MIN: the runner-up is the minimum once the winner's lane has swapped in its own second.
-                uint32_t lo, hi;
-                if (QPT == 2) {
-                    lo = min(kc[0], kc[1]);
-                    hi = max(kc[0], kc[1]);
-                } else {
-                    const uint32_t a0 = min(kc[0], kc[1]), b0 = max(kc[0], kc[1]);
-                    const uint32_t a1 = min(kc[QPT - 2], kc[QPT - 1]), b1 = max(kc[QPT - 2], kc[QPT - 1]);
-                    lo = min(a0, a1);
-                    hi = min(max(a0, a1), min(b0, b1));
-                }
-                const uint32_t m1 = __reduce_min_sync(0xFFFFFFFFu, lo);
-                const uint32_t m2 = __reduce_min_sync(0xFFFFFFFFu, lo == m1 ? hi : lo);
-                wstage[j] = make_uint2(m1, m2);   // warp-uniform value, every lane stores the same word: one wavefront
-            }
-            __syncwarp();
-            // lane j now merges train (g + j) into the CTA's column state.  The atomicMin chain keeps the two
-            // smallest of all keys ever offered (keys are unique): whatever loses slot .x is offered to slot .y.
-            if (lane < gn) {
-                const uint2 w = wstage[lane];
-                if (w.x != KEY_NONE) {
-                    uint2* cs = &col[c * K1_CHUNK + g + lane];
-                    const uint32_t old = atomicMin(&cs->x, w.x);
-                    atomicMin(&cs->y, max(old, w.x));
-                    if (w.y != KEY_NONE) atomicMin(&cs->y, w.y);
-                }
-            }
-            __syncwarp();
-        }
-        __syncthreads();
-    }
-
-#pragma unroll
-    for (int u = 0; u < QPT; ++u) {
-        const int q = tile.qb * QTILE + u * K1_THREADS + tid;
-        if (q < pr.n1) pr.rowpart[(size_t)tile.tb * pr.n1 + q] = make_uint2(k1[u], k2[u]);
-    }
-    uint2* cp = pr.colpart + (size_t)tile.qb * pr.n2 + t0;
-    for (int i = tid; i < nt; i += K1_THREADS) cp[i] = col[i];
-}
-
-typedef void (*K1Fn)(const MatchProblem*, const MatchTile*);
-
-// tuning knob PLSTVO_K1_VARIANT = "<queries per thread><popc per distance><min blocks per SM>"; default = measured best
-static int k1_variant_code() {
-    static const int code = [] {
-        const char* v = getenv("PLSTVO_K1_VARIANT");
-        return v ? atoi(v) : 253;
-    }();
-    return code;
-}
-
-int k1_queries_per_tile() { return K1_THREADS * ((k1_variant_code() / 100 == 4) ? 4 : 2); }
-
-static K1Fn k1_variant() {
-    switch (k1_variant_code()) {
-        case 254: return (K1Fn)hamming_knn2_kernel<5, 4, 2>;
-        case 263: return (K1Fn)hamming_knn2_kernel<6, 3, 2>;
-        case 243: return (K1Fn)hamming_knn2_kernel<4, 3, 2>;
-        case 452: return (K1Fn)hamming_knn2_kernel<5, 2, 4>;
-        case 462: return (K1Fn)hamming_knn2_kernel<6, 2, 4>;
-        case 442: return (K1Fn)hamming_knn2_kernel<4, 2, 4>;
-        case 453: return (K1Fn)hamming_knn2_kernel<5, 3, 4>;
-        default: return (K1Fn)hamming_knn2_kernel<5, 3, 2>;
-    }
-}
-
-cudaError_t launch_hamming_knn2(const MatchProblem* problems, const MatchTile* tiles, int n_tiles,
-                                int max_tsplit, cudaStream_t stream) {
-    if (n_tiles <= 0) return cudaSuccess;
-    const size_t smem = k1_smem_bytes(max_tsplit);
-    static size_t configured[64] = {};
-    K1Fn fn = k1_variant();
-    cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(fn), smem, configured);
-    if (e != cudaSuccess) return e;
-    fn<<<n_tiles, K1_THREADS, smem, stream>>>(problems, tiles);
-    return cudaGetLastError();
-}
 
 __global__ void __launch_bounds__(256) match_finalize_kernel(const MatchProblem* __restrict__ problems,
                                                              int32_t* __restrict__ counts) {
@@ -254,7 +35,7 @@ cudaError_t launch_match_finalize(const MatchProblem* problems, int n_problems, 
     return cudaGetLastError();
 }
 
-// ---- POPC issue-rate micro-benchmark (the integer roofline the matcher is held against) -------------
+// ---- POPC issue-rate micro-benchmark (plstvo_popc_rate) ---------------------------------------------
 __global__ void __launch_bounds__(256) popc_bench_kernel(uint32_t* out, int iters) {
     uint32_t x0 = threadIdx.x * 2654435761u + blockIdx.x, x1 = x0 ^ 0x9E3779B9u, x2 = x0 + 0x7F4A7C15u,
              x3 = x1 * 3u, x4 = x0 ^ 0x12345u, x5 = x1 + 77u, x6 = x2 ^ 0xABCDEFu, x7 = x3 + 1234567u;

@@ -1,22 +1,16 @@
-// match_finalize.cuh — merge of K1's tile partials, ratio test and mutual filter; shared by the standalone
+// match_finalize.cuh — ratio test and mutual filter on K1's merged partials; shared by the standalone
 // finalize kernel (match.cu) and the fused per-pair kernel K2 (solve.cu).
 #pragma once
 #include "common.cuh"
 
 namespace plstvo {
 
-// ---- merge of the tile partials + ratio test + mutual filter ---------------------------------------
+// ---- ratio test + mutual filter ----------------------------------------------------------------------
 // (src/matching.cpp:50-61 and :76-86)
 __device__ __forceinline__ bool ratio_accept(uint32_t a, uint32_t b, float nnr) {
     // matches_[idx][0].distance < matches_[idx][1].distance * nnr, all float (src/matching.cpp:54);
     // no second neighbour (n2 < 2: UB in the reference) -> no match
     return b != KEY_NONE && (float)(a >> 16) < __fmul_rn((float)(b >> 16), nnr);
-}
-
-__device__ __forceinline__ void merge_top2(uint32_t& a, uint32_t& b, const uint2 c) {
-    b = min(b, max(a, c.x));
-    a = min(a, c.x);
-    b = min(b, c.y);  // c.y > c.x >= a: it can only compete for the second place
 }
 
 // m21: 16-bit entries (an index is < 65535 = PLSTVO_MAX_FEATURES; 0xFFFF = no match), so that the largest admissible frame
@@ -46,35 +40,19 @@ __device__ __forceinline__ int match_finalize_block(const MatchProblem& pr, uint
         return 0;
     }
     const bool dist_form = pr.n1 <= (int)M21_DIST;
-    if (pr.nqb == 1 && pr.ntb == 1) {   // one partial per row / column (the tensor-core matcher): plain streaming loops, unrolled
-                                        // so that several of their independent loads are in flight per thread
+    // one partial per row / column: plain streaming loops, unrolled so that several of their independent loads are in
+    // flight per thread
 #pragma unroll 4
-        for (int t = tid; t < pr.n2; t += nth) {
-            const uint2 c = pr.colpart[t];
-            m21[t] = ratio_accept(c.x, c.y, pr.nnr) ? m21_entry(c.x, dist_form) : M21_NONE;
-        }
-        __syncthreads();
-#pragma unroll 4
-        for (int q = tid; q < pr.n1; q += nth) {
-            const uint2 c = pr.rowpart[q];
-            int32_t i2 = ratio_accept(c.x, c.y, pr.nnr) ? (int32_t)(c.x & 0xFFFFu) : -1;
-            if (pr.best_lr && i2 >= 0 && !m21_is_mutual(m21[i2], q, c.x, dist_form)) i2 = -1;
-            pr.m12[q] = i2;
-            count += (i2 >= 0);
-        }
-        return count;
-    }
     for (int t = tid; t < pr.n2; t += nth) {
-        uint32_t a = KEY_NONE, b = KEY_NONE;
-        for (int qb = 0; qb < pr.nqb; ++qb) merge_top2(a, b, pr.colpart[(size_t)qb * pr.n2 + t]);
-        m21[t] = ratio_accept(a, b, pr.nnr) ? (uint16_t)(a & 0xFFFFu) : M21_NONE;
+        const uint2 c = pr.colpart[t];
+        m21[t] = ratio_accept(c.x, c.y, pr.nnr) ? m21_entry(c.x, dist_form) : M21_NONE;
     }
     __syncthreads();
+#pragma unroll 4
     for (int q = tid; q < pr.n1; q += nth) {
-        uint32_t a = KEY_NONE, b = KEY_NONE;
-        for (int tb = 0; tb < pr.ntb; ++tb) merge_top2(a, b, pr.rowpart[(size_t)tb * pr.n1 + q]);
-        int32_t i2 = ratio_accept(a, b, pr.nnr) ? (int32_t)(a & 0xFFFFu) : -1;
-        if (pr.best_lr && i2 >= 0 && (int)m21[i2] != q) i2 = -1;
+        const uint2 c = pr.rowpart[q];
+        int32_t i2 = ratio_accept(c.x, c.y, pr.nnr) ? (int32_t)(c.x & 0xFFFFu) : -1;
+        if (pr.best_lr && i2 >= 0 && !m21_is_mutual(m21[i2], q, c.x, dist_form)) i2 = -1;
         pr.m12[q] = i2;
         count += (i2 >= 0);
     }

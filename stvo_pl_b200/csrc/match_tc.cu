@@ -19,8 +19,8 @@
 //                      (which 16-column group / which lane the best came from);
 //   tc_resolve_kernel  merges the per-block partials, converts to distances and recovers the best neighbour's index by
 //                      re-evaluating the <= 16 tagged candidates with XOR + POPC (exact; ties resolved to the lowest index
-//                      as OpenCV does), emitting the same packed keys (dist << 16 | index) K1's popcount form emits, so
-//                      everything downstream (ratio test, mutual filter, K2) is unchanged.
+//                      as OpenCV does), emitting packed keys (dist << 16 | index) whose unsigned order is OpenCV's
+//                      (distance, index) order, which the ratio test, the mutual filter and K2 read.
 // Integer-exact end to end: the bit-exact parity tests of the matcher are the acceptance test.
 #include <cuda_fp16.h>
 
@@ -129,16 +129,6 @@ __device__ __forceinline__ uint32_t hfma2u(uint32_t a, uint32_t b, uint32_t c) {
     asm("fma.rn.f16x2 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
     return d;
 }
-__device__ __forceinline__ uint32_t hfma2relu(uint32_t a, uint32_t b, uint32_t c) {   // max(0, a * b + c)
-    uint32_t d;
-    asm("fma.rn.relu.f16x2 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
-__device__ __forceinline__ uint32_t hadd2u(uint32_t a, uint32_t b) {
-    uint32_t d;
-    asm("add.rn.f16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
-    return d;
-}
 __device__ __forceinline__ uint32_t swap16(uint32_t a) { return __byte_perm(a, a, 0x1032); }
 __device__ __forceinline__ uint32_t sel32(uint32_t mask, uint32_t a, uint32_t b) { return (mask & a) | (~mask & b); }   // one LOP3
 __device__ __forceinline__ uint32_t h2u_lo(uint32_t p) {   // low half (an integer-valued f16 >= 0) -> uint32
@@ -152,24 +142,17 @@ __device__ __forceinline__ uint32_t h2u_hi(uint32_t p) {
     return d;
 }
 
-// "no value" sentinel: -1024 (finite, so that the FMA-pipe form of the update stays exact: |x - y| <= 1280 < 2048)
+// "no value" sentinel: -1024, below every dot value (>= -256)
 constexpr uint32_t NEG2 = 0xE400E400u;
-constexpr uint32_t H2_NEG1 = 0xBC00BC00u, H2_NEGHALF = 0xB800B800u, H2_128 = 0x58005800u, H2_511 = 0x5FFC5FFCu;
+constexpr uint32_t H2_NEGHALF = 0xB800B800u, H2_128 = 0x58005800u, H2_511 = 0x5FFC5FFCu;
 // (best, second) dot values packed (lo, hi) -> distances d = (256 - v) / 2 (exact), "none" (sentinel) -> 511
 __device__ __forceinline__ uint32_t dots_to_dist(uint32_t pv) { return hmin2u(hfma2u(pv, H2_NEGHALF, H2_128), H2_511); }
 
-// running top-2 update with one new packed value; ALU-pipe form (3 min/max) and FMA-pipe form (5 HFMA2 / HADD2):
-//   t = relu(v - k1); k1 += t; m = v - t (= min(k1, v)); k2 += relu(m - k2)        (all values integers, exact in f16)
+// running top-2 update with one new packed value: 3 min/max
 __device__ __forceinline__ void top2_alu(uint32_t& k1, uint32_t& k2, uint32_t v) {
     const uint32_t t = hmin2u(k1, v);
     k1 = hmax2u(k1, v);
     k2 = hmax2u(k2, t);
-}
-__device__ __forceinline__ void top2_fma(uint32_t& k1, uint32_t& k2, uint32_t v) {
-    const uint32_t t = hfma2relu(k1, H2_NEG1, v);
-    const uint32_t m = hfma2u(t, H2_NEG1, v);
-    k1 = hadd2u(k1, t);
-    k2 = hadd2u(k2, hfma2relu(k2, H2_NEG1, m));
 }
 // two new values at once: 5 ops (3 HMNMX2 + 2 VHMNMX)
 __device__ __forceinline__ void top2_pair(uint32_t& k1, uint32_t& k2, uint32_t a, uint32_t b) {
@@ -204,7 +187,6 @@ static_assert(TC_SMEM_USED + 1024 <= 227 * 1024, "tc_hamming_kernel: shared memo
 
 size_t tc_smem_bytes() { return (size_t)TC_SMEM_USED + 1024; }
 
-template <int NF>   // NF: column-state registers per 16-register chunk updated on the FMA pipe (0 .. 16)
 #ifndef TC_MAXNREG
 #define TC_MAXNREG 0
 #endif
@@ -373,10 +355,7 @@ tc_hamming_kernel(const TcProblem* __restrict__ problems, const TcItem* __restri
                     ta = sel32(hne2mask(ra1, olda), (uint32_t)((2 * c) * 0x00010001u), ta);
                     tb = sel32(hne2mask(rb1, oldb), (uint32_t)((2 * c + 1) * 0x00010001u), tb);
 #pragma unroll
-                    for (int i = 0; i < 16; ++i) {
-                        if (i < NF) top2_fma(c1[c * 16 + i], c2[c * 16 + i], v[i]);
-                        else top2_alu(c1[c * 16 + i], c2[c * 16 + i], v[i]);
-                    }
+                    for (int i = 0; i < 16; ++i) top2_alu(c1[c * 16 + i], c2[c * 16 + i], v[i]);
                 };
                 if (nvalid == CW && (t + 1) * TC_ROWS <= pr.n1 && debug_tile == nullptr) {
                     // full tile of a full block (the common case): no per-chunk branches, the next chunk's TMEM load is in
@@ -507,42 +486,24 @@ tc_hamming_kernel(const TcProblem* __restrict__ problems, const TcItem* __restri
     }
 }
 
-static int tc_nf() {   // tuning knob: how many of the 16 column registers per chunk use the FMA-pipe update
-    static const int nf = [] {
-        const char* v = getenv("PLSTVO_TC_NF");
-        return v ? atoi(v) : 0;
-    }();
-    return nf;
-}
-
 cudaError_t launch_tc_hamming(const TcProblem* problems, const TcItem* items_a, int n_a, const TcItem* items_b, int n_b,
                               int* sched, int grid, __half* debug_tile, cudaStream_t stream) {
     const int n_items = n_a + n_b;
     if (n_items <= 0) return cudaSuccess;
-    typedef void (*Fn)(const TcProblem*, const TcItem*, int, const TcItem*, int, int*, __half*);
-    Fn fn;
-    switch (tc_nf()) {
-        case 4: fn = tc_hamming_kernel<4>; break;
-        case 6: fn = tc_hamming_kernel<6>; break;
-        case 8: fn = tc_hamming_kernel<8>; break;
-        case 10: fn = tc_hamming_kernel<10>; break;
-        case 12: fn = tc_hamming_kernel<12>; break;
-        default: fn = tc_hamming_kernel<0>; break;
-    }
-    static size_t configured[8][64] = {};
+    static size_t configured[64] = {};
     const size_t smem = tc_smem_bytes();
-    cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(fn), smem, configured[(tc_nf() / 2) & 7]);
+    cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(tc_hamming_kernel), smem, configured);
     if (e != cudaSuccess) return e;
     if (grid > n_items) grid = n_items;
     if (getenv("PLSTVO_TC_DIAG")) {
         cudaFuncAttributes fa;
         int occ = -1;
-        cudaFuncGetAttributes(&fa, reinterpret_cast<const void*>(fn));
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, TC_THREADS, smem);
+        cudaFuncGetAttributes(&fa, reinterpret_cast<const void*>(tc_hamming_kernel));
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, tc_hamming_kernel, TC_THREADS, smem);
         fprintf(stderr, "[tc diag] regs %d, maxThreadsPerBlock %d, static smem %zu, local %zu, dynamic smem %zu, occupancy %d\n",
                 fa.numRegs, fa.maxThreadsPerBlock, fa.sharedSizeBytes, fa.localSizeBytes, smem, occ);
     }
-    fn<<<grid, TC_THREADS, smem, stream>>>(problems, items_a, n_a, items_b, n_b, sched, debug_tile);
+    tc_hamming_kernel<<<grid, TC_THREADS, smem, stream>>>(problems, items_a, n_a, items_b, n_b, sched, debug_tile);
     return cudaGetLastError();
 }
 

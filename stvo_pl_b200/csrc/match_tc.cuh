@@ -12,8 +12,8 @@ constexpr int TC_TILE_BYTES = TC_ROWS * 256;    // 128 rows x 256 e4m3 bytes, sw
 #define TC_EPILOGUE_WARPS 8
 #endif
 // epilogue warps: 8 (two per scheduler, 128 accumulator columns each) or 16 (four per scheduler, 64 columns each: 96 registers per
-// thread).  Measured on 512 C2 pairs: 8 warps 0.627 ms; 16 warps 0.664 ms, 0.625 ms with half of the column updates on the FMA pipe
-// (PLSTVO_TC_NF=8) — no gain, so 8 stays the default and -DTC_EPILOGUE_WARPS=16 remains a build option.
+// thread).  Measured on 512 C2 pairs: 8 warps 0.627 ms; 16 warps 0.664 ms, 0.625 ms with half of the column updates moved to the FMA
+// pipe (a variant since removed) — no gain, so 8 stays the default and -DTC_EPILOGUE_WARPS=16 remains a build option.
 constexpr int TC_EW = TC_EPILOGUE_WARPS;
 constexpr int TC_CW = 1024 / TC_EW;             // accumulator columns per epilogue warp = trains per row-partial block
 constexpr int TC_XSTAGES = TC_EW == 16 ? 3 : 4; // query tiles in flight (shared memory ring; 16 warps need the room for their scratch)
@@ -48,7 +48,7 @@ cudaError_t launch_tc_expand(const TcSide* sides, int n_sides, int max_tiles, cu
 // items_a then items_b form the work list (long items first); sched: two zeroed ints per concurrently running launch
 cudaError_t launch_tc_hamming(const TcProblem* problems, const TcItem* items_a, int n_a, const TcItem* items_b, int n_b,
                               int* sched, int grid, __half* debug_tile, cudaStream_t stream);
-// writes MatchProblem::rowpart[0][n1] / colpart[0][n2] (ntb = nqb = 1) in K1's packed-key format
+// writes MatchProblem::rowpart[n1] / colpart[n2] as packed keys (dist << 16 | index)
 cudaError_t launch_tc_resolve(const MatchProblem* mps, const TcProblem* tps, int n_problems, int slices, cudaStream_t stream);
 
 }  // namespace plstvo

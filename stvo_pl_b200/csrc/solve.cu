@@ -1,5 +1,5 @@
 // solve.cu — K2: one persistent CTA per frame pair does everything after the distance tiles:
-//   A. merge K1's partials, ratio test, mutual filter        (src/matching.cpp:50-61, :76-86)
+//   A. ratio test and mutual filter on K1's partials         (src/matching.cpp:50-61, :76-86)
 //   B. build matched_pt / matched_ls in ascending prev index  (src/stereoFrameHandler.cpp:144-152, :167-179)
 //      as structure-of-arrays in shared memory (coalesced, conflict-free), with the per-feature constants of the
 //      evaluator (sqrt(sigma2), the line-overlap coefficients) computed once
@@ -1395,7 +1395,7 @@ __device__ void finalize_pose(State& st, const PlPrior* prior, const Feat& f, in
         }
 }
 
-// Phases A and B of the per-pair work: finish the matching (merge K1's partials, ratio test, mutual filter -> m12) and build
+// Phases A and B of the per-pair work: finish the matching (ratio test and mutual filter on K1's partials -> m12) and build
 // matched_pt / matched_ls in ascending prev index as SoA (f), or copy the caller's explicit lists (mode 1).  Block-wide.
 // where the streamed solver wants the fp32 records of the lists (gn_stream.cuh "records"); on = false: fp64 lists only (K2)
 struct RecordSink {
@@ -1452,7 +1452,7 @@ __device__ void build_matched_lists(const SolveParams& prm, int pair, State& st,
     const int tid = threadIdx.x, nth = blockDim.x, lane = tid & 31, warp = tid >> 5, nw = nth >> 5;
     const PlConfig& cfg = prm.cfg;
     if (prm.mode == 0) {
-        // ---- A. finish the matching: merge partials, ratio test, mutual filter -> m12 (global) ----
+        // ---- A. finish the matching: ratio test, mutual filter -> m12 (global) ----
         const MatchProblem pp = prm.problems[2 * pair], pl = prm.problems[2 * pair + 1];
         match_finalize_block(pp, reinterpret_cast<uint16_t*>(sortbuf));
         __syncthreads();

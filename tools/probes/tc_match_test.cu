@@ -118,7 +118,7 @@ int main(int argc, char** argv) {
         max_tiles = std::max(max_tiles, std::max((q.n1 + 127) / 128, (q.n2 + 127) / 128));
         tps[p] = {ex + q.e1 * TC_TILE_BYTES, ex + q.e2 * TC_TILE_BYTES, q.n1, q.n2, rowp + q.rowp, colp + q.colp};
         MatchProblem m{};
-        m.d1 = d1 + q.o1 * 32; m.d2 = d2 + q.o2 * 32; m.n1 = q.n1; m.n2 = q.n2; m.nqb = 1; m.ntb = 1; m.enabled = 1;
+        m.d1 = d1 + q.o1 * 32; m.d2 = d2 + q.o2 * 32; m.n1 = q.n1; m.n2 = q.n2; m.enabled = 1;
         m.rowpart = rowpart + q.rowpart; m.colpart = colpart + q.colpart; m.nnr = nnr; m.best_lr = 1;
         mps[p] = m;
     }
