@@ -10,17 +10,20 @@
 //   tc_hamming_kernel  persistent, warp-specialised: producer warp (bulk copies + mbarriers), one MMA-issuing thread
 //                      (tcgen05.mma kind::f8f6f4, 128 x 128 x 32 per instruction, f16 accumulators in TMEM: every partial
 //                      sum is an integer of magnitude <= 256, exact in f16), eight epilogue warps reading TMEM with
-//                      tcgen05.ld ... .pack::16b: two columns per register, so the top-2 update of BOTH directions
-//                      costs 3 packed min/max per two distances and direction:
-//                        row direction   (query -> trains): thread = query row, fold over the columns in registers;
-//                        column direction (train -> queries): element-wise running top-2 over the row tiles in
-//                                         registers, one cross-lane reduction per work item (not per tile).
-//                      Keys carry no indices in the hot loop: only (best, second) VALUES and a small candidate tag
-//                      (which 16-column group / which lane the best came from);
-//   tc_resolve_kernel  merges the per-block partials, converts to distances and recovers the best neighbour's index by
-//                      re-evaluating the <= 16 tagged candidates with XOR + POPC (exact; ties resolved to the lowest index
-//                      as OpenCV does), emitting packed keys (dist << 16 | index) whose unsigned order is OpenCV's
-//                      (distance, index) order, which the ratio test, the mutual filter and K2 read.
+//                      tcgen05.ld ... .pack::16b: two columns per register.  The hot loop folds only MAXIMA:
+//                        row direction   (query -> trains): thread = query row; per 16-column group the packed maximum
+//                                         of 8 registers (4 three-input max) is the best of two "sets" (the 8 columns of
+//                                         one parity), and a running top-2 over set maxima keeps the best set's tag;
+//                        column direction (train -> queries): one packed max per register and row tile (each thread's
+//                                         best per column), one cross-lane reduction per work item (not per tile).
+//                      Keys carry no indices: the best value, the second over the OTHER sets / lanes (an upper bound
+//                      of the second distance) and the best set / lane as a tag;
+//   tc_resolve_kernel  merges the per-block partials and converts to distances.  Where the ratio test could pass against
+//                      the bound, it re-evaluates the tagged set (8 trains) or lane (queries tag + 128 i) with XOR + POPC:
+//                      the exact second distance is min(bound, second within the set / lane), and the scan gives the best
+//                      neighbour's index (ties resolved to the lowest index as OpenCV does).  It emits packed keys
+//                      (dist << 16 | index) whose unsigned order is OpenCV's (distance, index) order, which the ratio test,
+//                      the mutual filter and K2 read.
 // Integer-exact end to end: the bit-exact parity tests of the matcher are the acceptance test.
 #include <cuda_fp16.h>
 
@@ -154,12 +157,10 @@ __device__ __forceinline__ void top2_alu(uint32_t& k1, uint32_t& k2, uint32_t v)
     k1 = hmax2u(k1, v);
     k2 = hmax2u(k2, t);
 }
-// two new values at once: 5 ops (3 HMNMX2 + 2 VHMNMX)
-__device__ __forceinline__ void top2_pair(uint32_t& k1, uint32_t& k2, uint32_t a, uint32_t b) {
-    const uint32_t hi = hmax2u(a, b), lo = hmin2u(a, b);
-    const uint32_t t = hmin2u(k1, hi);
-    k2 = hmax2u(hmax2u(k2, lo), t);
-    k1 = hmax2u(hmax2u(k1, a), b);
+// maximum of 8 packed registers: 4 VHMNMX
+__device__ __forceinline__ uint32_t hmax8(const uint32_t* v) {
+    const uint32_t a = hmax2u(hmax2u(v[0], v[1]), v[2]), b = hmax2u(hmax2u(v[3], v[4]), v[5]);
+    return hmax2u(hmax2u(hmax2u(a, b), v[6]), v[7]);
 }
 
 // shared-memory operand descriptor: K-major, 128-byte swizzle, 8-row groups 1024 B apart (SBO), version 1
@@ -333,29 +334,28 @@ tc_hamming_kernel(const TcProblem* __restrict__ problems, const TcItem* __restri
             const int blk = item.yblk * (256 / CW) + gq;      // CW-column block index of this group
             const int ycol0 = blk * CW;
             const int nvalid = min(CW, pr.n2 - ycol0);        // <= 0: nothing for this group
-            uint32_t c1[NREG], c2[NREG];
+            uint32_t c1[NREG];   // column direction: per register and half, the best value this lane has seen
 #pragma unroll
-            for (int i = 0; i < NREG; ++i) c1[i] = c2[i] = NEG2;
+            for (int i = 0; i < NREG; ++i) c1[i] = NEG2;
 
             for (int t = 0; t < nxt; ++t) {
                 mbar_wait(&t_full[as], aph);
                 tc_fence_after();
                 const int x = t * TC_ROWS + q * 32 + lane;
                 const bool xvalid = x < pr.n1;
-                // two independent row chains: A = registers 0..7 (16-column group 2c), B = registers 8..15 (group 2c + 1)
+                // row direction: a "set" is the 8 columns of one parity in a 16-column group; each half of a group maximum
+                // is one set's maximum.  Two independent chains keep a running top-2 over set maxima and the group the
+                // maximum last rose in: A = registers 0..7 (group 2c), B = registers 8..15 (group 2c + 1)
                 uint32_t ra1 = NEG2, ra2 = NEG2, rb1 = NEG2, rb2 = NEG2, ta = 0, tb = 0;
                 const uint32_t tad = tmem_base + ((uint32_t)(q * 32) << 16) + as * 256 + gq * CW;
                 auto fold = [&](const uint32_t (&v)[16], const int c) {
                     const uint32_t olda = ra1, oldb = rb1;
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        top2_pair(ra1, ra2, v[2 * i], v[2 * i + 1]);
-                        top2_pair(rb1, rb2, v[8 + 2 * i], v[8 + 2 * i + 1]);
-                    }
+                    top2_alu(ra1, ra2, hmax8(v));
+                    top2_alu(rb1, rb2, hmax8(v + 8));
                     ta = sel32(hne2mask(ra1, olda), (uint32_t)((2 * c) * 0x00010001u), ta);
                     tb = sel32(hne2mask(rb1, oldb), (uint32_t)((2 * c + 1) * 0x00010001u), tb);
 #pragma unroll
-                    for (int i = 0; i < 16; ++i) top2_alu(c1[c * 16 + i], c2[c * 16 + i], v[i]);
+                    for (int i = 0; i < 16; ++i) c1[c * 16 + i] = hmax2u(c1[c * 16 + i], v[i]);
                 };
                 if (nvalid == CW && (t + 1) * TC_ROWS <= pr.n1 && debug_tile == nullptr) {
                     // full tile of a full block (the common case): no per-chunk branches, the next chunk's TMEM load is in
@@ -399,7 +399,8 @@ tc_hamming_kernel(const TcProblem* __restrict__ problems, const TcItem* __restri
                 if (lane == 0) mbar_arrive(&t_empty[as]);
                 if (++as == TC_ASTAGES) { as = 0; aph ^= 1; }
                 if (xvalid && nvalid > 0) {
-                    // chains, then the even- and odd-column streams; everything packed, the result sits in the low halves
+                    // chains, then the even- and odd-column sets; everything packed, the result sits in the low halves:
+                    // the best value, the second over the other sets, the best set as group << 1 | parity
                     const uint32_t m1 = hmax2u(ra1, rb1), m2 = hmax2u(hmax2u(hmin2u(ra1, rb1), ra2), rb2);
                     const uint32_t tg = sel32(hgt2mask(rb1, ra1), tb, ta);
                     const uint32_t s1 = swap16(m1), s2 = swap16(m2), st = swap16(tg);
@@ -410,9 +411,10 @@ tc_hamming_kernel(const TcProblem* __restrict__ problems, const TcItem* __restri
                 }
             }
 
-            // ---- column direction: reduce the element-wise state over the 128 threads of the group ----
+            // ---- column direction: reduce the lane maxima over the 128 threads of the group ----
             // per warp: transpose 16 registers at a time through shared memory; lane L folds register (L & 15) over
             // source lanes 16 (L >> 4) .. +15, the two halves meet by shuffle; then the four quarters merge per column.
+            // The result: the best value, the second over the other lanes, the best lane (query row mod 128)
 #pragma unroll
             for (int p = 0; p < NCH; ++p) {
                 const int j = lane & 15, hl = lane >> 4;
@@ -429,12 +431,6 @@ tc_hamming_kernel(const TcProblem* __restrict__ problems, const TcItem* __restri
                     id = sel32(hne2mask(nm, m1), (uint32_t)((hl * 16 + kk) * 0x00010001u), id);
                     m1 = nm;
                 }
-                __syncwarp();
-#pragma unroll
-                for (int i = 0; i < 16; ++i) scr[i * 33 + lane] = c2[p * 16 + i];
-                __syncwarp();
-#pragma unroll
-                for (int kk = 0; kk < 16; ++kk) m2 = hmax2u(m2, scr[j * 33 + hl * 16 + kk]);
                 __syncwarp();
                 // halves: lanes L and L ^ 16 hold the same register over the other 16 source lanes
                 const uint32_t o1 = __shfl_xor_sync(0xFFFFFFFFu, m1, 16), o2 = __shfl_xor_sync(0xFFFFFFFFu, m2, 16),
@@ -516,14 +512,39 @@ __device__ __forceinline__ int hamming256(const uint4& a0, const uint4& a1, cons
            __popc(a1.y ^ b1.y) + __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
 }
 
+// exact (best, second) distance from a over the rows j0, j0 + stride, ... (fewer than count of them, below n) of desc;
+// i1 = the lowest of those rows at the best distance
+__device__ __forceinline__ void scan_top2(const uint4& a0, const uint4& a1, const uint8_t* desc, int j0, int stride, int count,
+                                          int n, int& s1, int& s2, int& i1) {
+    s1 = s2 = 512;
+    i1 = -1;
+    for (int i = 0, j = j0; i < count && j < n; ++i, j += stride) {
+        const int h = hamming256(a0, a1, desc + (size_t)j * 32);
+        if (h < s1) { s2 = s1; s1 = h; i1 = j; }
+        else s2 = min(s2, h);
+    }
+}
+// an accepted tie (nnr > 1) or a best the candidates did not hold: lowest index at distance d among all n rows, as OpenCV
+// orders them
+__device__ __forceinline__ int first_at(const uint4& a0, const uint4& a1, const uint8_t* desc, int n, int d) {
+    for (int j = 0; j < n; ++j)
+        if (hamming256(a0, a1, desc + (size_t)j * 32) == d) return j;
+    return 0;
+}
+
+// The partials carry the best distance and an upper bound of the second: the second over the other candidate sets (rows) or
+// lanes (columns).  The exact second is min(bound, second within the best set / lane).  When the ratio test already fails
+// against the bound it fails against the exact second too (d2 <= bound), so the bound is written as k2 and nothing is
+// re-evaluated; ratio_accept (match_finalize.cuh), the only reader of k2, decides the same.  Otherwise the best set / lane is
+// re-evaluated with XOR + POPC, which gives the exact second and the index.
 __global__ void __launch_bounds__(256) tc_resolve_kernel(const MatchProblem* __restrict__ mps, const TcProblem* __restrict__ tps) {
     const MatchProblem mp = mps[blockIdx.x];
     if (!mp.enabled) return;
     const TcProblem tp = tps[blockIdx.x];
     const int nyh = (mp.n2 + TC_CW - 1) / TC_CW, nxt = (mp.n1 + TC_ROWS - 1) / TC_ROWS;   // row partials: one per TC_CW-train block
     const int slice = blockIdx.y, nslices = gridDim.y;
-    // partial word: best distance (9 bits) | second distance << 9 (511 = none) | candidate tag << 18
-    // queries: top-2 trains over the 128-train blocks (lowest block wins a tie: its indices are lower)
+    // partial word: best distance (9 bits) | second bound << 9 (511 = none) | candidate tag << 18
+    // queries: merge over the TC_CW-train blocks (lowest block wins a tie: its indices are lower)
     for (int x = slice * blockDim.x + threadIdx.x; x < mp.n1; x += nslices * blockDim.x) {
         uint32_t b1 = 511, b2 = 511, btag = 0;
         int bh = 0;
@@ -537,58 +558,45 @@ __global__ void __launch_bounds__(256) tc_resolve_kernel(const MatchProblem* __r
         uint32_t k2 = KEY_NONE;
         int idx = 0;
         if (mp.n2 >= 2) {
-            const int d2 = (int)b2;
-            k2 = ((uint32_t)d2 << 16) | 0xFFFEu;
+            int d2 = (int)b2;
             if ((float)d1 < __fmul_rn((float)d2, mp.nnr)) {
+                // the tagged set: 8 trains of one parity in one 16-column group
                 const uint4 a0 = __ldg(reinterpret_cast<const uint4*>(mp.d1 + (size_t)x * 32)),
                             a1 = __ldg(reinterpret_cast<const uint4*>(mp.d1 + (size_t)x * 32) + 1);
-                idx = -1;
-                if (d1 != d2) {   // unique best: it is one of the 8 tagged trains (16-column group, one parity)
-                    const int base = bh * TC_CW + (int)((btag >> 1) & 7u) * 16 + (int)(btag & 1u);
-                    for (int i = 0; i < 8 && idx < 0; ++i) {
-                        const int j = base + 2 * i;
-                        if (j < mp.n2 && hamming256(a0, a1, mp.d2 + (size_t)j * 32) == d1) idx = j;
-                    }
-                }
-                if (idx < 0) {   // tie accepted (nnr > 1): lowest index among all trains, as OpenCV orders them
-                    for (int j = 0; j < mp.n2 && idx < 0; ++j)
-                        if (hamming256(a0, a1, mp.d2 + (size_t)j * 32) == d1) idx = j;
-                    if (idx < 0) idx = 0;
-                }
+                const int base = bh * TC_CW + (int)((btag >> 1) & 7u) * 16 + (int)(btag & 1u);
+                int s1, s2, i1;
+                scan_top2(a0, a1, mp.d2, base, 2, 8, mp.n2, s1, s2, i1);
+                d2 = min(d2, s2);
+                if ((float)d1 < __fmul_rn((float)d2, mp.nnr)) idx = d1 != d2 && s1 == d1 ? i1 : first_at(a0, a1, mp.d2, mp.n2, d1);
             }
+            k2 = ((uint32_t)d2 << 16) | 0xFFFEu;
         }
         mp.rowpart[x] = make_uint2(((uint32_t)d1 << 16) | (uint32_t)idx, k2);
     }
-    // trains: top-2 queries
+    // trains: the best lane's queries are rows tag + 128 i
     for (int y = slice * blockDim.x + threadIdx.x; y < mp.n2; y += nslices * blockDim.x) {
         const uint32_t e = __ldg(&tp.colp[y]);
         const int d1 = (int)(e & 511u);
         uint32_t k2 = KEY_NONE;
         int idx = 0;
         if (mp.n1 >= 2) {
-            const int d2 = (int)((e >> 9) & 511u);
-            k2 = ((uint32_t)d2 << 16) | 0xFFFEu;
+            int d2 = (int)((e >> 9) & 511u);
             if ((float)d1 < __fmul_rn((float)d2, mp.nnr)) {
                 const uint4 a0 = __ldg(reinterpret_cast<const uint4*>(mp.d2 + (size_t)y * 32)),
                             a1 = __ldg(reinterpret_cast<const uint4*>(mp.d2 + (size_t)y * 32) + 1);
-                idx = -1;
-                if (d1 != d2 && mp.n1 <= (int)M21_DIST) {
-                    // unique best: WHICH query it is does not matter to the mutual filter (match_finalize.cuh: a query whose
-                    // nearest train is y at distance d1 is that query) — no candidate is re-evaluated
-                    idx = (int)KEY_IDX_UNRESOLVED;
-                } else if (d1 != d2) {   // (frames beyond 65024 rows) one of the queries the tagged epilogue thread saw (row = tag mod 128)
-                    const int t = (int)((e >> 18) & 127u);
-                    for (int i = 0; i < nxt && idx < 0; ++i) {
-                        const int j = t + i * TC_ROWS;
-                        if (j < mp.n1 && hamming256(a0, a1, mp.d1 + (size_t)j * 32) == d1) idx = j;
-                    }
-                }
-                if (idx < 0) {
-                    for (int j = 0; j < mp.n1 && idx < 0; ++j)
-                        if (hamming256(a0, a1, mp.d1 + (size_t)j * 32) == d1) idx = j;
-                    if (idx < 0) idx = 0;
+                int s1, s2, i1;
+                scan_top2(a0, a1, mp.d1, (int)((e >> 18) & 127u), TC_ROWS, nxt, mp.n1, s1, s2, i1);
+                d2 = min(d2, s2);
+                if ((float)d1 < __fmul_rn((float)d2, mp.nnr)) {
+                    if (d1 != d2 && s1 == d1)
+                        // unique best: up to 65024 rows WHICH query it is does not matter to the mutual filter
+                        // (match_finalize.cuh: a query whose nearest train is y at distance d1 is that query)
+                        idx = mp.n1 <= (int)M21_DIST ? (int)KEY_IDX_UNRESOLVED : i1;
+                    else
+                        idx = first_at(a0, a1, mp.d1, mp.n1, d1);
                 }
             }
+            k2 = ((uint32_t)d2 << 16) | 0xFFFEu;
         }
         mp.colpart[y] = make_uint2(((uint32_t)d1 << 16) | (uint32_t)idx, k2);
     }

@@ -33,8 +33,10 @@ struct TcProblem {
     const uint8_t* xe;    // expanded queries  (desc1): ceil(n1 / 128) tiles
     const uint8_t* ye;    // expanded trains   (desc2): ceil(n2 / 128) tiles
     int32_t n1, n2;
-    uint32_t* rowp;       // [ceil(n2 / TC_CW)][n1]: best distance | second << 9 (511 = none) | tag << 18 (16-column group, parity)
-    uint32_t* colp;       // [n2]:                 best | second << 9 | tag << 18 (query row mod 128)
+    // partials: best distance | second << 9 (511 = none) | tag << 18, where "second" is the second over the other candidate
+    // sets (rows) or lanes (columns), an upper bound of the exact second distance that tc_resolve_kernel refines
+    uint32_t* rowp;       // [ceil(n2 / TC_CW)][n1]: tag = best set (16-column group << 1 | parity: 8 trains)
+    uint32_t* colp;       // [n2]:                 tag = best lane (query row mod 128)
 };
 
 // one work item of the persistent kernel: all query tiles of a problem against 256 trains

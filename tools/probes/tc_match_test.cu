@@ -204,8 +204,15 @@ int main(int argc, char** argv) {
                 }
                 const uint2 g = out[a];
                 bool ok = (g.x >> 16) == (k1 >> 16);
-                if (nb >= 2) ok = ok && (g.y >> 16) == (k2 >> 16); else ok = ok && g.y == 0xFFFFFFFFu;
                 const bool acc = nb >= 2 && (float)(k1 >> 16) < (float)(k2 >> 16) * nnr;
+                // a rejected row / column may carry an upper bound of the second distance instead of the exact one: the
+                // decision must agree, the second itself only where the ratio test accepts
+                if (nb >= 2) {
+                    const bool got_acc = g.y != 0xFFFFFFFFu && (float)(g.x >> 16) < (float)(g.y >> 16) * nnr;
+                    ok = ok && got_acc == acc && (!acc || (g.y >> 16) == (k2 >> 16));
+                } else {
+                    ok = ok && g.y == 0xFFFFFFFFu;
+                }
                 // column direction: a unique nearest query is left unresolved (index field 0xFFFD): the mutual filter works on
                 // the distance alone (match_finalize.cuh)
                 const bool unresolved = dir == 1 && (g.x & 0xFFFF) == 0xFFFDu && (k1 >> 16) != (k2 >> 16) && nb <= 0xFE00;
